@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the MRFP hot path (BASELINE.json metric) — one JSON line on stdout.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 A "step" is one forward+backward pass of the whole MRFP path over one batch of synthetic stem / layer1
 features at BASELINE config[1] shapes (per GPU: batch 8, 768x768 crop -> 64ch and 256ch @192x192):
@@ -45,7 +45,33 @@ def parse():
     ap.add_argument("--steps", type=int, default=20)
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the outputs and gradients of the last one as DIR/<name>.npy "
+                         "(float32; arrays of more than 2^20 elements as the same seeded sample of 2^20 on every run)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
+    return args
+
+
+DUMP_SAMPLES = 1 << 20
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes every array as out_dir/<name>.npy in float32: whole if it has at most DUMP_SAMPLES elements, otherwise the
+    elements at DUMP_SAMPLES flat indices drawn without replacement by numpy's PCG64 seeded with 0, in ascending order —
+    the same positions on every run, so two builds can be compared output for output (at most 4 MB per array)."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        t = t.detach()
+        if t.numel() > DUMP_SAMPLES:
+            idx = np.sort(np.random.default_rng(0).choice(t.numel(), DUMP_SAMPLES, replace=False))
+            t = t.reshape(-1)[torch.from_numpy(idx).to(t.device)]
+        np.save(os.path.join(out_dir, name + ".npy"), t.float().cpu().numpy())
 
 
 # ----------------------------------------------------------------------------------------------------------
@@ -374,8 +400,9 @@ def run_ours(args):
         sampler.start()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
-    for _ in range(args.steps):
+    for _ in range(args.steps - 1):
         step(xp, f2, dec1_up, g_x, g_dec, g_f2)
+    last = step(xp, f2, dec1_up, g_x, g_dec, g_f2)
     e1.record()
     sync_all()
     ms = torch.tensor([e0.elapsed_time(e1)], device=dev)
@@ -386,6 +413,10 @@ def run_ours(args):
         sampler.join(timeout=2)
     total_ms = float(ms.item())
     value = world * n * args.steps / (total_ms * 1e-3)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, dict(zip(("x", "dec2", "np_plus_layer1", "grad_xp", "grad_layer1", "grad_dec1"), last),
+                                             grad_final2_weight=final2.weight.grad, grad_final2_bias=final2.bias.grad))
+    del last
     # round 1's step definition, same timing rules
     for _ in range(3):
         step_r1(xp, f2, dec1_up, g_x, g_dec_r1, g_f2)
@@ -438,7 +469,7 @@ def run_ours(args):
                 h.copy_(d, non_blocking=True)
             out_done[b].record(s_out)
 
-    e2e_steps = max(4, min(args.steps, 40))          # --steps steps (~25 ms each: PCIe-bound); the fill / drain of the three-stage pipeline is inside the region
+    e2e_steps = args.steps                           # ~25 ms each: PCIe-bound; the fill / drain of the three-stage pipeline is inside the region
     for i in range(4):                               # warm-up: both buffer sets twice (first-touch of the pinned pages, copy-engine set-up)
         e2e_step(i)
     cur.wait_stream(s_out)

@@ -68,6 +68,45 @@ def fill_state_dict(model, seed: int):
             t.copy_(torch.from_numpy(v.astype(np.float32)))
 
 
+def hrfp_gx_both(g, tag: str):
+    """Gradient into xp of both HRFP outputs from the hrfp.npz fixture.  The backward is linear in the upstream
+    gradients, so the fixture keeps only the two single-output gradients; their sum matches the reference's joint
+    backward to 6e-7 of max |.| (fp32 summation order), far inside every tolerance it is checked at."""
+    return g[f"{tag}_gx_out"] + g[f"{tag}_gx_dec"]
+
+
+# Eval-path cases of the host module on CPU: name -> (trunk, fill_state_dict seed, input shape).  Eval mode runs no
+# MRFP branch, so these pin the trunk and head wiring (tests/test_model.py, tests/golden/make_golden_hosts.py).
+HOST_EVAL_CASES = {"resnet50": ("resnet-50", 5, (2, 3, 64, 64)),
+                   "resnet101_trunk": ("resnet-101", 6, (2, 3, 64, 64)),
+                   "mobilenetv2": ("mobilenetv2", 9, (2, 3, 96, 160)),
+                   "shufflenetv2": ("shufflenetv2", 9, (2, 3, 96, 160))}
+
+
+def host_eval_case(name: str):
+    """(model, output) of one HOST_EVAL_CASES entry: weights from fill_state_dict, U[0,255) pixels from a seeded torch
+    generator.  The output is the logits, or for resnet101_trunk the layer2 feature (all three InstanceNorm sites).
+    Evaluated in float64: an fp32 run moves by up to 1.4e-5 of max |.| with the CPU's kernels and thread count."""
+    import torch
+    from mrfp_b200.model import MRFPPlus
+    trunk, seed, shape = HOST_EVAL_CASES[name]
+    m = MRFPPlus(19, trunk=trunk, criterion=torch.nn.CrossEntropyLoss(ignore_index=255))
+    fill_state_dict(m, seed)
+    m.double().eval()
+    x = torch.rand(shape, generator=torch.Generator().manual_seed(seed)).double() * 255
+    with torch.no_grad():
+        out = m.layer2(m.layer1(m._stem(x))) if name == "resnet101_trunk" else m(x, training=False)
+    return m, out
+
+
+def host_state_dict_digest(model) -> str:
+    """sha256 over the names and shapes of the host's state_dict entries (the HRFP layers left out), in state_dict order."""
+    import hashlib
+    from mrfp_b200.model import HRFP_CONVS, HRFP_BNS
+    lines = [f"{k} {list(v.shape)}" for k, v in model.state_dict().items() if k.split(".")[0] not in HRFP_CONVS + HRFP_BNS]
+    return hashlib.sha256("\n".join(lines).encode()).hexdigest()
+
+
 def make_in_case(seed: int, shape):
     """Inputs of one InstanceNorm2d(affine)+ReLU case: pre-norm features of both signs with channel-varying offsets,
     gamma ~ N(1, 0.3) (some negative via a sign flip), beta ~ N(0, 0.3), upstream gradient ~ N(0, 1)."""

@@ -10,7 +10,6 @@ if ROOT not in sys.path:
 
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA device (run on the B200 box with -m gpu)")
-    config.addinivalue_line("markers", "refonly: needs /root/reference (build container only)")
 
 
 def pytest_collection_modifyitems(config, items):
@@ -20,10 +19,6 @@ def pytest_collection_modifyitems(config, items):
     except Exception:
         has_gpu = False
     skip_gpu = pytest.mark.skip(reason="no CUDA device")
-    skip_ref = pytest.mark.skip(reason="/root/reference not present")
-    has_ref = os.path.isfile("/root/reference/deepv3.py")
     for item in items:
         if "gpu" in item.keywords and not has_gpu:
             item.add_marker(skip_gpu)
-        if "refonly" in item.keywords and not has_ref:
-            item.add_marker(skip_ref)

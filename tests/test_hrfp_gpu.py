@@ -7,7 +7,7 @@ import pytest
 import torch
 
 from oracle import mrfp_oracle as O
-from tests.common import GOLDEN, make_hrfp_params, make_feat
+from tests.common import GOLDEN, hrfp_gx_both, make_hrfp_params, make_feat
 
 pytestmark = pytest.mark.gpu
 
@@ -94,7 +94,7 @@ def test_vs_reference_fixture(tag, mode):
     out, dec, gx, bns, _ = _run(xp, ws, gs, h, w, mode, g1, g2)
     _check(out, g[f"{tag}_ocout"], mode, "fwd")
     _check(dec, g[f"{tag}_ocout_dec"].astype(np.float32), mode, "fwd", floor=2e-3)         # fixture stored as fp16
-    _check(gx, g[f"{tag}_gx_both"], mode, "bwd")
+    _check(gx, hrfp_gx_both(g, tag), mode, "bwd")
     for k in range(8):
         rtol = {0: 1e-4, 1: 2e-3, 2: 2e-2}[mode]
         assert np.allclose(bns[k].running_mean.cpu().numpy(), g[f"{tag}_rm{k}"], rtol=rtol, atol=rtol)

@@ -1,5 +1,6 @@
-"""Drop-in module: state_dict compatibility, eval-path equality with the reference (container only) and the
-full training forward/backward against a fixture produced by the reference itself."""
+"""Drop-in module: state_dict compatibility, eval-path equality with the reference (stored vectors,
+tests/golden/make_golden_hosts.py) and the full training forward/backward against a fixture produced by the reference
+itself."""
 import json
 import os
 import random
@@ -8,7 +9,7 @@ import numpy as np
 import pytest
 import torch
 
-from tests.common import GOLDEN, make_hrfp_params, make_draws, fill_state_dict
+from tests.common import GOLDEN, make_hrfp_params, make_draws, fill_state_dict, host_eval_case, host_state_dict_digest
 
 
 def _criterion():
@@ -54,20 +55,24 @@ def test_eval_forward_needs_no_kernels_and_is_deterministic():
     assert a.shape == (1, 19, 64, 64) and torch.equal(a, b)
 
 
-@pytest.mark.refonly
+def _check_host_eval(name):
+    """One tests.common.HOST_EVAL_CASES case against tests/golden/hosts_eval.npz (tests/golden/make_golden_hosts.py): the
+    sampled outputs and sum |.| to the tolerance the reference's own modules were held to, the state_dict names and shapes
+    exactly."""
+    g = np.load(os.path.join(GOLDEN, "hosts_eval.npz"))
+    m, out = host_eval_case(name)
+    y = out.double().numpy()
+    amax = float(g[f"{name}_absmax"])
+    assert list(y.shape) == list(g[f"{name}_shape"])
+    assert np.allclose(y.ravel()[g[f"{name}_idx"]], g[f"{name}_val"], rtol=1e-5, atol=1e-5 * amax)
+    assert abs(np.abs(y).max() - amax) <= 1e-5 * amax
+    assert abs(np.abs(y).sum() - float(g[f"{name}_abssum"])) <= 1e-5 * float(g[f"{name}_abssum"])
+    assert host_state_dict_digest(m) == str(g[f"{name}_digest"])
+    return m
+
+
 def test_eval_forward_equals_reference_on_cpu():
-    from oracle.ref_shim import load_reference
-    from mrfp_b200.model import MRFPPlus
-    ref = load_reference().MRFPPlus(19, criterion=_criterion())
-    mine = MRFPPlus(19, criterion=_criterion())
-    fill_state_dict(ref, 5)
-    mine.load_state_dict(ref.state_dict(), strict=True)
-    ref.eval(); mine.eval()
-    x = torch.rand(2, 3, 64, 64) * 255
-    with torch.no_grad():
-        a = ref(x, training=False)
-        b = mine(x, training=False)
-    assert torch.allclose(a, b, rtol=1e-5, atol=1e-5 * a.abs().max().item())
+    _check_host_eval("resnet50")
 
 
 def _train_step(math_mode):
@@ -169,7 +174,6 @@ def test_gates_off_is_plain_deeplab_and_skips_hrfp():
 
 
 # ---- trunk="resnet-101" (SURVEY.md 8f-2, BASELINE config[3]): the reference's deep-stem ResNet-101 under the same hooks ----
-_R101_STEM = {"conv1": "layer0.0", "bn1": "layer0.1", "conv2": "layer0.3", "bn2": "layer0.4", "conv3": "layer0.6", "bn3": "layer0.7"}
 
 
 def test_resnet101_host_shapes():
@@ -187,33 +191,10 @@ def test_resnet101_host_shapes():
         MRFPPlus(19, trunk="resnet-18", criterion=_criterion())
 
 
-@pytest.mark.refonly
 def test_resnet101_trunk_equals_reference_resnet101_on_cpu():
-    """layer0..layer2 (all three InstanceNorm sites) against the reference's own network/Resnet.py resnet101."""
-    from oracle.ref_shim import load_reference
-    from mrfp_b200.model import MRFPPlus
-    load_reference()
-    from network import Resnet
-    ref = Resnet.resnet101(pretrained=False, wt_layer=[0, 0, 4, 4, 4, 0, 0])
-    mine = MRFPPlus(19, trunk="resnet-101", criterion=_criterion())
-    fill_state_dict(ref, 6)
-    sd = {}
-    for k, v in ref.state_dict().items():
-        head = k.split(".")[0]
-        if head in _R101_STEM:
-            sd[_R101_STEM[head] + k[len(head):]] = v
-        elif head.startswith("layer"):
-            sd[k] = v
-    missing, unexpected = mine.load_state_dict(sd, strict=False)
-    assert not unexpected
-    assert all(not k.startswith(("layer0", "layer1", "layer2", "layer3", "layer4")) for k in missing), missing
-    ref.eval(); mine.eval()
-    x = torch.rand(2, 3, 64, 64) * 255
-    with torch.no_grad():
-        r = ref.maxpool(ref.relu3(ref.bn3(ref.conv3(ref.relu2(ref.bn2(ref.conv2(ref.relu1(ref.bn1(ref.conv1(x))))))))))
-        r = ref.layer2(ref.layer1([r, []]))[0]
-        o = mine.layer2(mine.layer1(mine._stem(x)))
-    assert torch.allclose(r, o, rtol=1e-5, atol=1e-5 * r.abs().max().item())
+    """layer0..layer2 (all three InstanceNorm sites) of the ResNet-101 host, which carries the reference's
+    network/Resnet.py resnet101 (its conv1 / bn1 ... conv3 / bn3 stem as layer0.0 ... layer0.7)."""
+    _check_host_eval("resnet101_trunk")
 
 
 @pytest.mark.gpu
@@ -236,27 +217,11 @@ def test_resnet101_training_step_runs_all_branches():
 
 
 # ---- trunk="mobilenetv2" / "shufflenetv2" (SURVEY.md 8f-2, BASELINE config[4]) ----
-@pytest.mark.refonly
 @pytest.mark.parametrize("trunk", ["mobilenetv2", "shufflenetv2"])
 def test_mobile_hosts_load_the_reference_state_dict_and_match_its_eval_forward_on_cpu(trunk):
     """The host is state_dict-compatible with the reference's DeepV3Plus(trunk) (network/deepv3.py:103-556; its `dsn`
     auxiliary head aside) and evaluates to the same logits — eval mode has no MRFP, so this pins the trunk wiring."""
-    import importlib
-    from oracle.ref_shim import load_reference
-    from mrfp_b200.model import MRFPPlus, HRFP_CONVS, HRFP_BNS
-    load_reference()
-    nd = importlib.import_module("network.deepv3")
-    ref = nd.DeepV3Plus(19, trunk=trunk, criterion=None, variant="D16", args=None).eval()
-    mine = MRFPPlus(19, trunk=trunk, criterion=_criterion()).eval()
-    fill_state_dict(ref, 9)
-    sd = {k: v for k, v in ref.state_dict().items() if not k.startswith("dsn.")}
-    mk = {k for k in mine.state_dict() if k.split(".")[0] not in HRFP_CONVS + HRFP_BNS}
-    assert mk == set(sd)
-    mine.load_state_dict(sd, strict=False)
-    x = torch.rand(2, 3, 96, 160) * 255
-    with torch.no_grad():
-        a, b = ref(x), mine(x, training=False)
-    assert torch.allclose(a, b, rtol=1e-5, atol=1e-5 * a.abs().max().item())
+    mine = _check_host_eval(trunk)
     stem = {"mobilenetv2": 16, "shufflenetv2": 24}[trunk]
     assert mine.OClayer1.in_channels == stem and mine.OCdeclayer4.out_channels == stem
     assert mine.hrfp_scale == {"mobilenetv2": 2, "shufflenetv2": 1}[trunk]

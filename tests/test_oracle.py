@@ -8,7 +8,7 @@ import numpy as np
 import pytest
 
 from oracle import mrfp_oracle as O
-from tests.common import GOLDEN, make_hrfp_params, make_feat, make_draws
+from tests.common import GOLDEN, hrfp_gx_both, make_hrfp_params, make_feat, make_draws
 
 
 @pytest.fixture(scope="module")
@@ -134,7 +134,7 @@ def test_hrfp_forward_backward_vs_reference(g_hrfp, tag):
     g2 = rng.standard_normal(ocdec.shape).astype(np.float32).astype(np.float64)
     for key, (a, b) in {"gx_both": (g1, g2), "gx_out": (g1, None), "gx_dec": (None, g2)}.items():
         gx = O.hrfp_backward(a, b, ws64, gs64, saved)
-        refg = g_hrfp[f"{tag}_{key}"]
+        refg = hrfp_gx_both(g_hrfp, tag) if key == "gx_both" else g_hrfp[f"{tag}_{key}"]
         assert np.abs(gx - refg).max() <= 5e-4 * np.abs(refg).max(), key
     # BN buffer side effect (SURVEY §8 a-8)
     for k in range(8):
@@ -194,7 +194,8 @@ def test_torch_port_hrfp_vs_reference(g_hrfp):
     g2 = torch.from_numpy(rng.standard_normal(tuple(d.shape)).astype(np.float32))
     torch.autograd.backward([o, d], [g1, g2])
     assert np.abs(o.detach().numpy() - g_hrfp["sq_ocout"]).max() <= 1e-4 * np.abs(g_hrfp["sq_ocout"]).max()
-    assert np.abs(xp.grad.numpy() - g_hrfp["sq_gx_both"]).max() <= 1e-3 * np.abs(g_hrfp["sq_gx_both"]).max()
+    gx_both = hrfp_gx_both(g_hrfp, "sq")
+    assert np.abs(xp.grad.numpy() - gx_both).max() <= 1e-3 * np.abs(gx_both).max()
 
 
 @pytest.mark.parametrize("name", list("abcd"))
