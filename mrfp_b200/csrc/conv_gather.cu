@@ -97,8 +97,10 @@ __device__ __forceinline__ void ld8s(uint32_t a, float (&v)[8]) {
 //               replica, 0 where it has none (a pixel the down-sampling skipped receives no gradient)
 // each inside the image, 0 in the convolution's zero padding
 // ADD: 0 nothing joins the output; 1 a tensor of the output's shape is added in the epilogue (add tile by TMA); 2 a RANK-K
-// term joins as one more k-block of the accumulation: out += G[pixel][64] . W2T[cout][64]^T (the classifier tail's gradient,
-// tail_final2.cu) — its two operands travel through the weight ring: tmap_add describes G (N, H, W, 64), tmap_rkw W2T (cout, 64)
+// term joins as one more k-block of the accumulation: out += G[pixel][0:32] . W2T[cout][0:32]^T (the classifier tail's gradient,
+// tail_final2.cu) — its two operands travel through the weight ring: tmap_add describes G (N, H, W, 64), tmap_rkw W2T (cout, 64).
+// Two UMMA k-steps of 16 read columns 0..31 only: the tail takes <= 24 classes and leaves the columns beyond them zero
+// (include/mrfp_b200.h), so columns 32..63 are padding of the 128-byte rows and never enter the product
 template <int COUT, int MODE, int ADD, int MT>
 __global__ void __launch_bounds__(kGThreads, 1)
 conv3x3_gather_kernel(const __grid_constant__ CUtensorMap tmap_w, const __grid_constant__ CUtensorMap tmap_out,
@@ -760,7 +762,8 @@ extern "C" int mrfp_debug_conv3x3_gather_bwd(const void* y, const void* dA, int 
   return mrfp::conv3x3_gather_bwd(y, dA, OH, OW, lo_h, lo_w, host_lo_h, host_lo_w, max_rep, stats, gamma, acc, count, cin, wpack, out, N,
                                   H, W, cin, cout, dil, (cudaStream_t)stream, false, add_src, nullptr, nullptr);
 }
-// ... the stage-4 form with the rank-K term: g64 (N, H, W, 64) bf16 and w2t (cout, 64) bf16 (see conv3x3_gather_kernel, ADD == 2)
+// ... the stage-4 form with the rank-K term: g64 (N, H, W, 64) bf16 and w2t (cout, 64) bf16, of which columns 0..31 enter the
+// product (see conv3x3_gather_kernel, ADD == 2)
 extern "C" int mrfp_debug_conv3x3_gather_bwd_rk(const void* y, const void* dA, int OH, int OW, const int* lo_h, const int* lo_w,
                                                 const int* host_lo_h, const int* host_lo_w, const float* stats, const float* gamma,
                                                 const double* acc, double count, const void* wpack, void* out, int N, int H, int W,

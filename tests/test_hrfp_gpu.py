@@ -448,13 +448,18 @@ def test_tail_fused_through_the_classifier_equals_the_unfused_tail(geom):
     assert float((got.double() - ref).norm() / ref.norm()) <= 5e-3
 
 
-@pytest.mark.parametrize("geom", [(2, 96, 80, (24, 20), 19), (1, 96, 544, (24, 136), 7)])
-def test_rank_k_form_of_the_tail_gradient_in_the_full_chain(geom, monkeypatch):
+# the last geometry has a stage-4 plane of 50 x 44: neither a multiple of the dgrad's 16 x 8 tile on either axis
+@pytest.mark.parametrize("geom", [(2, 96, 80, (24, 20), 19), (1, 96, 544, (24, 136), 7), (2, 100, 88, (25, 20), 19)])
+@pytest.mark.parametrize("fuse", [3, 1, 0])
+@pytest.mark.parametrize("want_out", [True, False])
+def test_rank_k_form_of_the_tail_gradient_in_the_full_chain(geom, fuse, want_out, monkeypatch):
     """The gradient of OCout_dec out of the fused classifier tail is W2^T g (rank K): by default it joins the chain as its two
     factors and the stage-4 dgrad accumulates their product as one more k-block (mrfp_hrfp_tail_final2_bwd_rk + mrfp_hrfp_bwd_rk,
     conv_gather.cu ADD == 2) — against the materialised (N, h/2, w/2, 256) bf16 tensor added in that dgrad's epilogue
-    (MRFP_TAIL_RANKK=0) and against the unfused tail; full chain, so that the stage-4 dgrad runs."""
-    from mrfp_b200.hrfp import hrfp_chain, hrfp_plus_add_upsampled, hrfp_plus_final2
+    (MRFP_TAIL_RANKK=0) and against the unfused tail.  Without the fused BN backward (fuse bit 1 off: fuse 0, 1) the stage-4
+    dgrad is the tap kernel and the product is expanded into the dA buffer first; in the encoder-only backward
+    (want_out=False, no stage-4 dgrad) the expansion is dA_3 itself."""
+    from mrfp_b200.hrfp import hrfp_chain, hrfp_plus_add_upsampled, hrfp_plus_final2, tail_final2_supported
     n, h, w, lo, k = geom
     xh, xw = math.ceil(h / 4), math.ceil(w / 4)
     ws, gs = make_hrfp_params(81)
@@ -470,11 +475,16 @@ def test_rank_k_form_of_the_tail_gradient_in_the_full_chain(geom, monkeypatch):
         monkeypatch.setenv("MRFP_TAIL_RANKK", "0" if name == "materialised" else "1")
         final2.zero_grad(set_to_none=True)
         xa = xp.clone().requires_grad_(True); da = d_lo.clone().requires_grad_(True)
-        x, dec = hrfp_chain(xa, convs, bns, h, w, math_mode=2, lazy_dec=True, update_running_stats=False)
+        x, dec = hrfp_chain(xa, convs, bns, h, w, want_out=want_out, math_mode=2, lazy_dec=True, update_running_stats=False,
+                            fuse=fuse)
+        assert dec.plan.fuse == fuse
+        if name != "unfused":
+            assert tail_final2_supported(da, final2, dec)
         out = hrfp_plus_final2(da, final2, dec) if name != "unfused" else final2(hrfp_plus_add_upsampled(da, dec))
-        torch.autograd.backward([x, out], [gx, g])
+        torch.autograd.backward([x, out] if want_out else [out], [gx, g] if want_out else [g])
         res[name] = [t.detach().clone() for t in (out, da.grad, final2.weight.grad, xa.grad)]
     rel = lambda a, b: float((a.double() - b.double()).norm() / b.double().norm())
+    print({nm: rel(res["rank_k"][i], res["materialised"][i]) for i, nm in enumerate(("dec2", "g_dec1", "g_W2", "g_xp"))})
     for i, nm in enumerate(("dec2", "g_dec1", "g_W2")):
         assert rel(res["rank_k"][i], res["materialised"][i]) <= 1e-5, nm      # the same kernels up to the atomics' order
     assert rel(res["rank_k"][3], res["materialised"][3]) <= 2e-2              # one rounding instead of two on the way into dA_3
