@@ -8,21 +8,12 @@
 // pass and of the BN-backward reduce and apply passes on the bf16 path (521 / 573 / 675 us vs 550 / 720 / 850 us for the
 // LDG kernels; a single persistent ring per SM measured slower than both, profiles/README.md).
 #include "hrfp.cuh"
-#include "tma.cuh"
+#include "ptx.cuh"
 
 namespace mrfp {
 namespace {
 
-using namespace tma;
-
-__device__ __forceinline__ void unpack8(const uint4 r, float (&v)[8]) {
-  const uint32_t w[4] = {r.x, r.y, r.z, r.w};
-#pragma unroll
-  for (int i = 0; i < 4; ++i) {
-    v[2 * i] = __uint_as_float(w[i] << 16);
-    v[2 * i + 1] = __uint_as_float(w[i] & 0xffff0000u);
-  }
-}
+using namespace ptx;
 
 // U1[c] = sum mask*dA, U2[c] = sum mask*dA*y over all destination pixels; mask = [scale*y + shift > 0], y gathered.
 // Each CTA copies one item (a <= 20 KiB gradient segment + the gathered span of the conv-output row) into its own buffer,
@@ -177,13 +168,7 @@ bn_bwd_apply_bulk_kernel(const __nv_bfloat16* __restrict__ dA, const __nv_bfloat
         const float t = fmaf(r_scale[j], yv[j], r_shift[j]) > 0.f ? sd[j] : 0.f;
         o[j] = r_P[j] * t - cnt * fmaf(r_R[j], yv[j], r_Q[j]);
       }
-      uint32_t w[4];
-#pragma unroll
-      for (int i = 0; i < 4; ++i) {
-        const __nv_bfloat162 h = __floats2bfloat162_rn(o[2 * i], o[2 * i + 1]);
-        w[i] = *reinterpret_cast<const uint32_t*>(&h);
-      }
-      *reinterpret_cast<uint4*>(dY + ((long long)row * IW + x0 + x) * C + c) = make_uint4(w[0], w[1], w[2], w[3]);
+      *reinterpret_cast<uint4*>(dY + ((long long)row * IW + x0 + x) * C + c) = pack8(o);
       w0 = nw0; w1 = nw1;
     }
     __syncthreads();                                     // every read of the buffers precedes the next item's copies
@@ -234,11 +219,8 @@ bn_relu_resample_bulk_kernel(const __nv_bfloat16* __restrict__ y, __nv_bfloat16*
       unpack8(*reinterpret_cast<const uint4*>(smem_raw + ((size_t)j * C + c) * 2), v);
       uint32_t w[4];
 #pragma unroll
-      for (int i = 0; i < 4; ++i) {
-        const __nv_bfloat162 h = __floats2bfloat162_rn(fmaxf(fmaf(sc[2 * i], v[2 * i], sf[2 * i]), 0.f),
-                                                       fmaxf(fmaf(sc[2 * i + 1], v[2 * i + 1], sf[2 * i + 1]), 0.f));
-        w[i] = *reinterpret_cast<const uint32_t*>(&h);
-      }
+      for (int i = 0; i < 4; ++i)
+        w[i] = pack_bf16x2(fmaxf(fmaf(sc[2 * i], v[2 * i], sf[2 * i]), 0.f), fmaxf(fmaf(sc[2 * i + 1], v[2 * i + 1], sf[2 * i + 1]), 0.f));
       *reinterpret_cast<uint4*>(dst + (size_t)px * C) = make_uint4(w[0], w[1], w[2], w[3]);
       j = jn;
     }

@@ -30,7 +30,8 @@ __host__ __device__ inline size_t align_up(size_t v, size_t a) { return (v + a -
 // Programmatic dependent launch: every kernel of the HRFP chain is launched with the stream-serialisation attribute and
 // starts with pdl_sync().  The trigger lets the NEXT kernel be scheduled (block launch, barrier / TMEM set-up,
 // descriptor fetch) while this one is still running; the wait returns only when all prerequisite grids have
-// completed and flushed, so every global access behind it sees the same ordering as a plain stream launch.
+// completed and flushed, so every global access behind it sees the same ordering as a plain stream launch.  The trigger
+// is ptx::pdl_trigger() (ptx.cuh).
 __device__ __forceinline__ void pdl_sync() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
 // cudaFuncSetAttribute(MaxDynamicSharedMemorySize) once per (kernel, device): `flag` is a static of the call site
 #define MRFP_SMEM_OPT_IN(kern, bytes, device)                                                              \
@@ -90,6 +91,20 @@ __device__ __forceinline__ uint32_t bn_relu_x2(uint32_t v, uint64_t scale2, uint
   asm("cvt.rn.bf16x2.f32 %0, %1, %2;" : "=r"(p) : "f"(hi), "f"(lo));
   asm("max.bf16x2 %0, %1, %2;" : "=r"(p) : "r"(p), "r"(0u));
   return p;
+}
+
+// 8 consecutive bf16 values in a uint4 (value 2i in the low half of word i) <-> 8 floats; packing rounds to nearest even
+__device__ __forceinline__ void unpack8(const uint4& v, float (&f)[8]) {
+  const uint32_t w[4] = {v.x, v.y, v.z, v.w};
+#pragma unroll
+  for (int i = 0; i < 4; ++i) { f[2 * i] = __uint_as_float(w[i] << 16); f[2 * i + 1] = __uint_as_float(w[i] & 0xffff0000u); }
+}
+__device__ __forceinline__ uint32_t pack_bf16x2(float lo, float hi) {
+  const __nv_bfloat162 h = __floats2bfloat162_rn(lo, hi);
+  return *reinterpret_cast<const uint32_t*>(&h);
+}
+__device__ __forceinline__ uint4 pack8(const float (&f)[8]) {
+  return make_uint4(pack_bf16x2(f[0], f[1]), pack_bf16x2(f[2], f[3]), pack_bf16x2(f[4], f[5]), pack_bf16x2(f[6], f[7]));
 }
 
 __device__ __forceinline__ double warp_sum(double v) {

@@ -4,6 +4,7 @@
 // finalisation by the last CTA).
 #pragma once
 #include "hrfp.cuh"
+#include "ptx.cuh"
 
 namespace mrfp {
 namespace convk {
@@ -25,40 +26,21 @@ template <> struct Elem<float> {
   static constexpr CUtensorMapDataType kStoreType = CU_TENSOR_MAP_DATA_TYPE_FLOAT32;
 };
 
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(uint64_t* bar, uint32_t count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count));
-}
-__device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
-  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ void mbar_expect_tx(uint64_t* bar, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "WAIT_%=:\n\t"
-      "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n\t"
-      "@p bra DONE_%=;\n\t"
-      "bra WAIT_%=;\n\t"
-      "DONE_%=:\n\t}" ::"r"(smem_u32(bar)), "r"(parity) : "memory");
-}
 __device__ __forceinline__ void tma_load_4d(void* dst, const CUtensorMap* map, uint64_t* bar, int c0, int c1, int c2, int c3) {
   asm volatile("cp.async.bulk.tensor.4d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5, %6}], [%2];"
-               ::"r"(smem_u32(dst)), "l"(reinterpret_cast<uint64_t>(map)), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "r"(c2), "r"(c3)
+               ::"r"(ptx::smem_u32(dst)), "l"(reinterpret_cast<uint64_t>(map)), "r"(ptx::smem_u32(bar)), "r"(c0), "r"(c1), "r"(c2), "r"(c3)
                : "memory");
 }
 __device__ __forceinline__ void tma_load_2d(void* dst, const CUtensorMap* map, uint64_t* bar, int c0, int c1) {
   asm volatile("cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];"
-               ::"r"(smem_u32(dst)), "l"(reinterpret_cast<uint64_t>(map)), "r"(smem_u32(bar)), "r"(c0), "r"(c1) : "memory");
+               ::"r"(ptx::smem_u32(dst)), "l"(reinterpret_cast<uint64_t>(map)), "r"(ptx::smem_u32(bar)), "r"(c0), "r"(c1) : "memory");
 }
 __device__ __forceinline__ void tma_store_4d(const CUtensorMap* map, const void* src, int c0, int c1, int c2, int c3) {
   asm volatile("cp.async.bulk.tensor.4d.global.shared::cta.bulk_group [%0, {%2, %3, %4, %5}], [%1];"
-               ::"l"(reinterpret_cast<uint64_t>(map)), "r"(smem_u32(src)), "r"(c0), "r"(c1), "r"(c2), "r"(c3) : "memory");
+               ::"l"(reinterpret_cast<uint64_t>(map)), "r"(ptx::smem_u32(src)), "r"(c0), "r"(c1), "r"(c2), "r"(c3) : "memory");
 }
 __device__ __forceinline__ void umma_commit(uint64_t* bar) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar)) : "memory");
+  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(ptx::smem_u32(bar)) : "memory");
 }
 // D[tmem] (+)= A[smem] * B[smem]^T with fp32 accumulation, issued by one thread for the CTA
 template <typename T>
@@ -91,7 +73,7 @@ __device__ __forceinline__ void tmem_ld32(uint32_t taddr, uint32_t (&r)[32]) {
         "=r"(r[16]), "=r"(r[17]), "=r"(r[18]), "=r"(r[19]), "=r"(r[20]), "=r"(r[21]), "=r"(r[22]), "=r"(r[23]),
         "=r"(r[24]), "=r"(r[25]), "=r"(r[26]), "=r"(r[27]), "=r"(r[28]), "=r"(r[29]), "=r"(r[30]), "=r"(r[31])
       : "r"(taddr));
-  asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+  ptx::tcgen05_wait_ld();
 }
 __device__ __forceinline__ bool elect_one() {
   uint32_t pred;
@@ -99,23 +81,6 @@ __device__ __forceinline__ bool elect_one() {
   return pred != 0;
 }
 __device__ __forceinline__ void epi_bar_sync() { asm volatile("bar.sync 1, 128;" ::: "memory"); }
-// Explicit shared-space accesses by 32-bit address: the 1024-byte alignment of the dynamic shared memory goes through an
-// integer, after which the compiler treats derived pointers as generic (LD.E / ST.E on the shared window — correct, but with
-// the latency of the global path).  volatile asm keeps them ordered against the barriers around them.
-__device__ __forceinline__ void sts_v4(uint32_t a, uint32_t x, uint32_t y, uint32_t z, uint32_t w) {
-  asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(a), "r"(x), "r"(y), "r"(z), "r"(w) : "memory");
-}
-__device__ __forceinline__ void sts_f32(uint32_t a, float v) { asm volatile("st.shared.f32 [%0], %1;" ::"r"(a), "f"(v) : "memory"); }
-__device__ __forceinline__ uint32_t lds_u32(uint32_t a) {
-  uint32_t v;
-  asm volatile("ld.shared.b32 %0, [%1];" : "=r"(v) : "r"(a));
-  return v;
-}
-__device__ __forceinline__ float lds_f32(uint32_t a) {
-  float v;
-  asm volatile("ld.shared.f32 %0, [%1];" : "=f"(v) : "r"(a));
-  return v;
-}
 
 // Geometry of a CTA tile: MT sub-tiles of TH x TW = 128 output pixels (one TMEM lane per pixel), stacked vertically
 // (HMT = false, the tap kernel) or side by side (HMT = true, the gather kernel).
@@ -155,7 +120,7 @@ __device__ __forceinline__ void conv_epilogue(const EpiSmem& sm, uint32_t tmem_b
   constexpr bool kBf16 = sizeof(T) == 2;
   unsigned char* const sOut = sm.sOut;
   float* const s_wgt = sm.s_wgt;
-  const uint32_t s_wgt_u = smem_u32(sm.s_wgt);
+  const uint32_t s_wgt_u = ptx::smem_u32(sm.s_wgt);
   uint64_t* const tmem_full = sm.tmem_full;
   uint64_t* const tmem_empty = sm.tmem_empty;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -198,7 +163,7 @@ __device__ __forceinline__ void conv_epilogue(const EpiSmem& sm, uint32_t tmem_b
     const int t_ = rev ? num_tiles - 1 - t0_ : t0_;
     const int tw_ = t_ % tiles_w, th_ = (t_ / tiles_w) % tiles_h, n_ = t_ / (tiles_w * tiles_h);
     const int mt_ = jj_ / kChunks, j_ = jj_ % kChunks;
-    mbar_expect_tx(&sm.add_full[buf], kStageOutBytes);
+    ptx::mbar_expect_tx(&sm.add_full[buf], kStageOutBytes);
     tma_load_4d(sOut + buf * kStageOutBytes, tmap_add, &sm.add_full[buf], j_ * kChunkC, G::w0(tw_) + G::dw(mt_), G::h0(th_) + G::dh(mt_), n_);
   };
   if (ADD == 3 && leader) add_issue(blockIdx.x, 0, 0);
@@ -208,8 +173,8 @@ __device__ __forceinline__ void conv_epilogue(const EpiSmem& sm, uint32_t tmem_b
     const int tw = t % tiles_w, th = (t / tiles_w) % tiles_h, n = t / (tiles_w * tiles_h);
     const int h0 = G::h0(th), w0 = G::w0(tw);
     const int acc = it & 1;
-    mbar_wait(&tmem_full[acc], (it >> 1) & 1);
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+    ptx::mbar_wait(&tmem_full[acc], (it >> 1) & 1);
+    ptx::tcgen05_after_sync();
 #pragma unroll
     for (int jj = 0; jj < MT * kChunks; ++jj) {
       const int mt = jj / kChunks, j = jj % kChunks;
@@ -222,7 +187,7 @@ __device__ __forceinline__ void conv_epilogue(const EpiSmem& sm, uint32_t tmem_b
       if (ADD == 2) ad_ok = ad_nxt_ok;
       const int bsel = (MT * kChunks) % 2 == 0 ? (jj & 1) : ((it * MT * kChunks + jj) & 1);
       unsigned char* ob = sOut + bsel * kStageOutBytes;
-      const uint32_t ob_u = smem_u32(ob);
+      const uint32_t ob_u = ptx::smem_u32(ob);
       if (ADD == 3) {
         // the store of the previous chunk must have read the OTHER buffer before the next chunk's add tile lands in it
         if (leader) {
@@ -234,7 +199,7 @@ __device__ __forceinline__ void conv_epilogue(const EpiSmem& sm, uint32_t tmem_b
         if (leader) asm volatile("cp.async.bulk.wait_group.read 1;" ::: "memory");
       }
       epi_bar_sync();
-      if (stat_acc) sts_f32(s_wgt_u + 4u * (uint32_t)r, (float)(cnt_h[h0 + G::dh(mt) + hl] * cnt_w[w0 + G::dw(mt) + wl]));   // 0 outside the image (zero-padded tables)
+      if (stat_acc) ptx::sts_f32(s_wgt_u + 4u * (uint32_t)r, (float)(cnt_h[h0 + G::dh(mt) + hl] * cnt_w[w0 + G::dw(mt) + wl]));   // 0 outside the image (zero-padded tables)
       const uint32_t tcol = (uint32_t)((acc * MT + mt) * COUT + j * kChunkC);
       if constexpr (kBf16) {
 #pragma unroll
@@ -242,13 +207,12 @@ __device__ __forceinline__ void conv_epilogue(const EpiSmem& sm, uint32_t tmem_b
           uint32_t v[32];
           tmem_ld32(tmem_base + ((uint32_t)(q * 32) << 16) + tcol + (uint32_t)(half * 32), v);
           if (ADD == 3) {                        // this row's half of the add tile, from the buffer the sum goes back into
-            if (half == 0) mbar_wait(&sm.add_full[bsel], (uint32_t)(((it * MT * kChunks + jj) >> 1) & 1));
+            if (half == 0) ptx::mbar_wait(&sm.add_full[bsel], (uint32_t)(((it * MT * kChunks + jj) >> 1) & 1));
 #pragma unroll
             for (int c = 0; c < 4; ++c) {
               const int chunk = half * 4 + c;
-              uint32_t w4[4];
-              asm volatile("ld.shared.v4.b32 {%0, %1, %2, %3}, [%4];"
-                           : "=r"(w4[0]), "=r"(w4[1]), "=r"(w4[2]), "=r"(w4[3]) : "r"(ob_u + (uint32_t)(r * 128 + ((chunk ^ (r & 7)) << 4))));
+              const uint4 a4 = ptx::lds_v4(ob_u + (uint32_t)(r * 128 + ((chunk ^ (r & 7)) << 4)));
+              const uint32_t w4[4] = {a4.x, a4.y, a4.z, a4.w};
 #pragma unroll
               for (int i = 0; i < 4; ++i) {
                 v[c * 8 + 2 * i] = __float_as_uint(__uint_as_float(v[c * 8 + 2 * i]) + __uint_as_float(w4[i] << 16));
@@ -272,12 +236,9 @@ __device__ __forceinline__ void conv_epilogue(const EpiSmem& sm, uint32_t tmem_b
           for (int c = 0; c < 4; ++c) {          // four 16-byte chunks (8 channels each) per half
             uint32_t p[4];
 #pragma unroll
-            for (int i = 0; i < 4; ++i) {
-              const __nv_bfloat162 h2 = __floats2bfloat162_rn(__uint_as_float(v[c * 8 + 2 * i]), __uint_as_float(v[c * 8 + 2 * i + 1]));
-              p[i] = *reinterpret_cast<const uint32_t*>(&h2);
-            }
+            for (int i = 0; i < 4; ++i) p[i] = pack_bf16x2(__uint_as_float(v[c * 8 + 2 * i]), __uint_as_float(v[c * 8 + 2 * i + 1]));
             const int chunk = half * 4 + c;
-            sts_v4(ob_u + (uint32_t)(r * 128 + ((chunk ^ (r & 7)) << 4)), p[0], p[1], p[2], p[3]);
+            ptx::sts_v4(ob_u + (uint32_t)(r * 128 + ((chunk ^ (r & 7)) << 4)), p[0], p[1], p[2], p[3]);
           }
         }
       } else {
@@ -293,18 +254,18 @@ __device__ __forceinline__ void conv_epilogue(const EpiSmem& sm, uint32_t tmem_b
             o.z = __float_as_uint(__uint_as_float(o.z) + __uint_as_float(a4.z));
             o.w = __float_as_uint(__uint_as_float(o.w) + __uint_as_float(a4.w));
           }
-          sts_v4(ob_u + (uint32_t)(r * 128 + ((c ^ (r & 7)) << 4)), o.x, o.y, o.z, o.w);
+          ptx::sts_v4(ob_u + (uint32_t)(r * 128 + ((c ^ (r & 7)) << 4)), o.x, o.y, o.z, o.w);
         }
       }
       if (ADD == 2 && add_src != nullptr) {    // the single register set is free again: the next chunk's loads
         if (jj + 1 < MT * kChunks) add_fetch(t0, jj + 1); else add_fetch(t0 + gridDim.x, 0);
       }
       if (jj == MT * kChunks - 1) {       // all TMEM reads of this accumulator are done
-        asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+        ptx::tcgen05_before_sync();
         __syncwarp();
-        if (lane == 0) mbar_arrive(&tmem_empty[acc]);
+        if (lane == 0) ptx::mbar_arrive(&tmem_empty[acc]);
       }
-      asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+      ptx::fence_proxy_async_smem();
       epi_bar_sync();
       if (leader) {
         tma_store_4d(&tmap_out, ob, j * kChunkC, w0 + G::dw(mt), h0 + G::dh(mt), n);
@@ -318,8 +279,8 @@ __device__ __forceinline__ void conv_epilogue(const EpiSmem& sm, uint32_t tmem_b
 #pragma unroll 8
         for (int i = 0; i < 32; ++i) {
           const int row = pg * 32 + i;
-          const uint32_t w2 = lds_u32(col + (uint32_t)(row * 128 + ((ch ^ (row & 7)) << 4)));
-          const float wg = lds_f32(s_wgt_u + 4u * (uint32_t)row);
+          const uint32_t w2 = ptx::lds_u32(col + (uint32_t)(row * 128 + ((ch ^ (row & 7)) << 4)));
+          const float wg = ptx::lds_f32(s_wgt_u + 4u * (uint32_t)row);
           if constexpr (kBf16) {
             const float y0 = __uint_as_float(w2 << 16), y1 = __uint_as_float(w2 & 0xffff0000u);
             const float t0 = wg * y0, t1 = wg * y1;

@@ -32,6 +32,7 @@
 namespace mrfp {
 namespace {
 using namespace convk;
+using namespace ptx;
 
 constexpr int kGThreads = 448;
 constexpr int kGTileH = 16, kGSubW = 8;        // M sub-tile: 16 rows x 8 columns
@@ -65,29 +66,8 @@ struct GatherArgs {
 };
 
 __device__ __forceinline__ void prod_bar_sync() { asm volatile("bar.sync 2, 256;" ::: "memory"); }
-// explicit shared-space accesses by 32-bit address (see conv_common.cuh)
-__device__ __forceinline__ int lds32(uint32_t a) { int v; asm volatile("ld.shared.b32 %0, [%1];" : "=r"(v) : "r"(a)); return v; }
-__device__ __forceinline__ uint4 lds128(uint32_t a) {
-  uint4 v;
-  asm volatile("ld.shared.v4.b32 {%0, %1, %2, %3}, [%4];" : "=r"(v.x), "=r"(v.y), "=r"(v.z), "=r"(v.w) : "r"(a));
-  return v;
-}
-__device__ __forceinline__ void unpack8(const uint4& v, float (&f)[8]) {
-  const uint32_t w[4] = {v.x, v.y, v.z, v.w};
-#pragma unroll
-  for (int i = 0; i < 4; ++i) { f[2 * i] = __uint_as_float(w[i] << 16); f[2 * i + 1] = __uint_as_float(w[i] & 0xffff0000u); }
-}
-__device__ __forceinline__ uint4 pack8(const float (&f)[8]) {
-  uint32_t p[4];
-#pragma unroll
-  for (int i = 0; i < 4; ++i) {
-    const __nv_bfloat162 h2 = __floats2bfloat162_rn(f[2 * i], f[2 * i + 1]);
-    p[i] = *reinterpret_cast<const uint32_t*>(&h2);
-  }
-  return make_uint4(p[0], p[1], p[2], p[3]);
-}
 __device__ __forceinline__ void ld8s(uint32_t a, float (&v)[8]) {
-  const uint4 x = lds128(a), y = lds128(a + 16);
+  const uint4 x = lds_v4(a), y = lds_v4(a + 16);
   v[0] = __uint_as_float(x.x); v[1] = __uint_as_float(x.y); v[2] = __uint_as_float(x.z); v[3] = __uint_as_float(x.w);
   v[4] = __uint_as_float(y.x); v[5] = __uint_as_float(y.y); v[6] = __uint_as_float(y.z); v[7] = __uint_as_float(y.w);
 }
@@ -140,22 +120,22 @@ conv3x3_gather_kernel(const __grid_constant__ CUtensorMap tmap_w, const __grid_c
   const int npix = boxh * boxw;
 
   if (threadIdx.x == 0) {
-    asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(&tmap_w)) : "memory");
-    asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(&tmap_out)) : "memory");
-    if (ADD) asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(&tmap_add)) : "memory");
-    if (ADD == 2) asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(&tmap_rkw)) : "memory");
+    prefetch_tensormap(&tmap_w);
+    prefetch_tensormap(&tmap_out);
+    if (ADD) prefetch_tensormap(&tmap_add);
+    if (ADD == 2) prefetch_tensormap(&tmap_rkw);
     for (int i = 0; i < nA; ++i) { mbar_init(&full_a[i], kProducers); mbar_init(&empty_a[i], 1); }
     for (int i = 0; i < nB; ++i) { mbar_init(&full_b[i], 1); mbar_init(&empty_b[i], 1); }
     for (int i = 0; i < 2; ++i) { mbar_init(&tmem_full[i], 1); mbar_init(&tmem_empty[i], 4); mbar_init(&add_full[i], 1); }
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    mbar_fence_init();
   }
   if (warp == 1) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_ptr)), "n"(kTmemCols) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+    tmem_alloc<kTmemCols>(tmem_ptr);
+    tmem_relinquish();
   }
-  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+  tcgen05_before_sync();
   __syncthreads();
-  asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+  tcgen05_after_sync();
   const uint32_t tmem_base = *tmem_ptr;
   pdl_sync();                                 // set-up above overlaps the previous kernel's tail
 
@@ -193,7 +173,7 @@ conv3x3_gather_kernel(const __grid_constant__ CUtensorMap tmap_w, const __grid_c
         if (++bs == nB) { bs = 0; bph ^= 1; }
       }
     }
-    asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
+    pdl_trigger();
   } else if (warp == 1) {
     // ===================== MMA issuer (whole warp walks with warp-uniform values, one elected lane issues) ==========
     constexpr uint32_t idesc = (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(COUT >> 3) << 17) | ((128u >> 4) << 24);
@@ -206,7 +186,7 @@ conv3x3_gather_kernel(const __grid_constant__ CUtensorMap tmap_w, const __grid_c
     for (int t = blockIdx.x; t < num_tiles; t += gridDim.x, ++it) {
       const int acc = it & 1;
       mbar_wait(&tmem_empty[acc], ((it >> 1) & 1) ^ 1);
-      asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+      tcgen05_after_sync();
       const uint32_t d_tmem = tmem_u + (uint32_t)(acc * MT * COUT);
       for (int kc = 0; kc < nchunks; ++kc) {
         mbar_wait(&full_a[as], aph);
@@ -214,7 +194,7 @@ conv3x3_gather_kernel(const __grid_constant__ CUtensorMap tmap_w, const __grid_c
 #pragma unroll 3
         for (int tap = 0; tap < 9; ++tap) {
           mbar_wait(&full_b[bs], bph);
-          asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+          tcgen05_after_sync();
           if (elect_one()) {
             // the tap's view starts (ty * d * boxw + tx * d) box pixels into the halo tile; descriptors advance in 16-byte units
             const uint64_t da = da_stage + (uint64_t)(((tap / 3) * dil * boxw + (tap % 3) * dil) * 8);
@@ -241,7 +221,7 @@ conv3x3_gather_kernel(const __grid_constant__ CUtensorMap tmap_w, const __grid_c
         const int ws_ = bs;
         mbar_wait(&full_b[bs], bph);
         if (++bs == nB) { bs = 0; bph ^= 1; }
-        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+        tcgen05_after_sync();
         if (elect_one()) {
           // G tile as TMA wrote it: [16 rows][8 px][128 B], i.e. eight-pixel groups 1024 bytes apart (SBO = 64 x 16 bytes)
           const uint64_t dg = (1ull << 16) | (64ull << 32) | (1ull << 46) | (2ull << 61) |
@@ -321,18 +301,16 @@ conv3x3_gather_kernel(const __grid_constant__ CUtensorMap tmap_w, const __grid_c
             const int v = __shfl_up_sync(0xffffffffu, x, o);
             if (lane_ >= o) x += v;
           }
-          if (lane_ == 31) asm volatile("st.shared.b32 [%0], %1;" ::"r"(scan_u + 4u * (uint32_t)wid), "r"(x) : "memory");
+          if (lane_ == 31) sts_u32(scan_u + 4u * (uint32_t)wid, (uint32_t)x);
           prod_bar_sync();
           int before = carry, total = carry;
 #pragma unroll
           for (int i = 0; i < kProducers / 32; ++i) {
-            const int v = lds32(scan_u + 4u * (uint32_t)i);
+            const int v = (int)lds_u32(scan_u + 4u * (uint32_t)i);
             if (i < wid) before += v;
             total += v;
           }
-          if (p < npix)
-            asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};"
-                         ::"r"(tab + 16u * (uint32_t)p), "r"(oy), "r"(og), "r"(before + x - e), "r"(nh | (nw << 8)) : "memory");
+          if (p < npix) sts_v4(tab + 16u * (uint32_t)p, (uint32_t)oy, (uint32_t)og, (uint32_t)(before + x - e), (uint32_t)(nh | (nw << 8)));
           carry = total;
           prod_bar_sync();                       // the warp totals are reused by the next pass
         }
@@ -343,14 +321,14 @@ conv3x3_gather_kernel(const __grid_constant__ CUtensorMap tmap_w, const __grid_c
         const bool in = (unsigned)h < (unsigned)H && (unsigned)w < (unsigned)W;
         if constexpr (MODE == kGatherFwd) {
           const int off = in ? (n * ga.SH + ga.tab_h[h]) * ga.SW + ga.tab_w[w] : -1;
-          asm volatile("st.shared.b32 [%0], %1;" ::"r"(tab + 4u * (uint32_t)p), "r"(off) : "memory");
+          sts_u32(tab + 4u * (uint32_t)p, (uint32_t)off);
         } else {
           int oy = -1, og = 0;
           if (in) {
             const int dh = ga.tab_h[h], dw = ga.tab_w[w];
             if (ga.tab_h[h + 1] > dh && ga.tab_w[w + 1] > dw) { oy = (n * H + h) * W + w; og = (n * ga.SH + dh) * ga.SW + dw; }
           }
-          asm volatile("st.shared.v2.b32 [%0], {%1, %2};" ::"r"(tab + 8u * (uint32_t)p), "r"(oy), "r"(og) : "memory");
+          sts_v2(tab + 8u * (uint32_t)p, (uint32_t)oy, (uint32_t)og);
         }
       }
       prod_bar_sync();
@@ -376,30 +354,27 @@ conv3x3_gather_kernel(const __grid_constant__ CUtensorMap tmap_w, const __grid_c
 #pragma unroll
         for (int u = 0; u < U; ++u) {
           if (pl + kPxLanes * u < npix) {
-            const int off = lds32(tab + (uint32_t)(kEnt * kPxLanes * u));
+            const int off = (int)lds_u32(tab + (uint32_t)(kEnt * kPxLanes * u));
             const __nv_bfloat16* src = off >= 0 ? ga.y + (size_t)off * CIN + c0 : ga.y;
             // an identically-zero pixel: source size 0 zero-fills the 16 bytes
-            asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;"
-                         ::"r"(dst0 + (uint32_t)(kPxLanes * 128 * u)), "l"(src), "r"(off >= 0 ? 16 : 0) : "memory");
+            cp_async_cg16_zfill(dst0 + (uint32_t)(kPxLanes * 128 * u), src, off >= 0 ? 16u : 0u);
             if constexpr (kBwd) {
               if (off >= 0) {
-                const int og = lds32(tab + (uint32_t)(kEnt * kPxLanes * u) + 4u);
+                const int og = (int)lds_u32(tab + (uint32_t)(kEnt * kPxLanes * u) + 4u);
                 const __nv_bfloat16* gp = ga.g + (size_t)og * CIN + c0;
-                asm volatile("cp.async.cg.shared.global [%0], [%1], 16;"
-                             ::"r"(sG_u + my_off + (uint32_t)(kPxLanes * 128 * u)), "l"(gp) : "memory");
+                cp_async_cg16(sG_u + my_off + (uint32_t)(kPxLanes * 128 * u), gp);
                 if constexpr (MODE == kGatherBwdRep) {     // replicas (0,1), (1,0), (1,1) -> consecutive rows of the extras stage
-                  const int rep = lds32(tab + (uint32_t)(kEnt * kPxLanes * u) + 12u);
+                  const int rep = (int)lds_u32(tab + (uint32_t)(kEnt * kPxLanes * u) + 12u);
                   if (rep != (1 | (1 << 8))) {
                     const int nh = rep & 0xff, nw = rep >> 8;
-                    uint32_t ed = sE_u + (uint32_t)lds32(tab + (uint32_t)(kEnt * kPxLanes * u) + 8u) * 128u + (uint32_t)(piece << 4);
+                    uint32_t ed = sE_u + lds_u32(tab + (uint32_t)(kEnt * kPxLanes * u) + 8u) * 128u + (uint32_t)(piece << 4);
                     if (nw > 1) {
-                      asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(ed), "l"(gp + CIN) : "memory");
+                      cp_async_cg16(ed, gp + CIN);
                       ed += 128u;
                     }
                     if (nh > 1) {
-                      asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(ed), "l"(gp + (size_t)ga.SW * CIN) : "memory");
-                      if (nw > 1)
-                        asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(ed + 128u), "l"(gp + (size_t)ga.SW * CIN + CIN) : "memory");
+                      cp_async_cg16(ed, gp + (size_t)ga.SW * CIN);
+                      if (nw > 1) cp_async_cg16(ed + 128u, gp + (size_t)ga.SW * CIN + CIN);
                     }
                   }
                 }
@@ -412,7 +387,7 @@ conv3x3_gather_kernel(const __grid_constant__ CUtensorMap tmap_w, const __grid_c
         if (++i_as == nA) { i_as = 0; i_ph ^= 1; }
         ++i_item;
       }
-      asm volatile("cp.async.commit_group;" ::: "memory");     // one group per call, empty or not: uniform accounting
+      cp_async_commit();                         // one group per call, empty or not: uniform accounting
       return valid;
     };
     uint32_t vq0 = 0, vq1 = 0, vq2 = 0;          // live-pixel masks of the items in flight, oldest first
@@ -423,9 +398,9 @@ conv3x3_gather_kernel(const __grid_constant__ CUtensorMap tmap_w, const __grid_c
     for (int j = 0; j < nitems; ++j) {
       if (LA == 0) vq0 = issue_next();           // backward: copy, wait, transform — the MMAs of item j - 1 run meanwhile
       // item j is the oldest of the groups in flight
-      if (LA <= 1) asm volatile("cp.async.wait_group 0;" ::: "memory");
-      else if (LA == 2) asm volatile("cp.async.wait_group 1;" ::: "memory");
-      else asm volatile("cp.async.wait_group 2;" ::: "memory");
+      if (LA <= 1) cp_async_wait<0>();
+      else if (LA == 2) cp_async_wait<1>();
+      else cp_async_wait<2>();
       const uint32_t dst0 = sA_u + (uint32_t)(j_as * a_stage_bytes) + my_off;
       const uint32_t valid = vq0;
       if constexpr (MODE == kGatherFwd) {
@@ -441,7 +416,7 @@ conv3x3_gather_kernel(const __grid_constant__ CUtensorMap tmap_w, const __grid_c
 #pragma unroll
           for (int i = 0; i < 5; ++i) {
             v[i] = make_uint4(0u, 0u, 0u, 0u);
-            if (u0 + i < U && pl + kPxLanes * (u0 + i) < npix) v[i] = lds128(dst0 + (uint32_t)(kPxLanes * 128 * (u0 + i)));
+            if (u0 + i < U && pl + kPxLanes * (u0 + i) < npix) v[i] = lds_v4(dst0 + (uint32_t)(kPxLanes * 128 * (u0 + i)));
           }
 #pragma unroll
           for (int i = 0; i < 5; ++i) {
@@ -449,9 +424,7 @@ conv3x3_gather_kernel(const __grid_constant__ CUtensorMap tmap_w, const __grid_c
               uint4 o = make_uint4(bn_relu_x2(v[i].x, sc2[0], sh2[0]), bn_relu_x2(v[i].y, sc2[1], sh2[1]),
                                    bn_relu_x2(v[i].z, sc2[2], sh2[2]), bn_relu_x2(v[i].w, sc2[3], sh2[3]));
               if (!((valid >> (u0 + i)) & 1u)) o = make_uint4(0u, 0u, 0u, 0u);   // the convolution's zero padding stays zero
-              if (pl + kPxLanes * (u0 + i) < npix)
-                asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};"
-                             ::"r"(dst0 + (uint32_t)(kPxLanes * 128 * (u0 + i))), "r"(o.x), "r"(o.y), "r"(o.z), "r"(o.w) : "memory");
+              if (pl + kPxLanes * (u0 + i) < npix) sts_v4(dst0 + (uint32_t)(kPxLanes * 128 * (u0 + i)), o.x, o.y, o.z, o.w);
             }
           }
         }
@@ -468,8 +441,8 @@ conv3x3_gather_kernel(const __grid_constant__ CUtensorMap tmap_w, const __grid_c
           for (int i = 0; i < 3; ++i) {
             vy[i] = vg[i] = make_uint4(0u, 0u, 0u, 0u);
             if (u0 + i < U && ((valid >> (u0 + i)) & 1u)) {
-              vy[i] = lds128(dst0 + (uint32_t)(kPxLanes * 128 * (u0 + i)));
-              vg[i] = lds128(g0 + (uint32_t)(kPxLanes * 128 * (u0 + i)));
+              vy[i] = lds_v4(dst0 + (uint32_t)(kPxLanes * 128 * (u0 + i)));
+              vg[i] = lds_v4(g0 + (uint32_t)(kPxLanes * 128 * (u0 + i)));
             }
           }
 #pragma unroll
@@ -480,13 +453,13 @@ conv3x3_gather_kernel(const __grid_constant__ CUtensorMap tmap_w, const __grid_c
               float cnt = 1.f;
               if constexpr (MODE == kGatherBwdRep) {             // the other replicas, in the order (0,1), (1,0), (1,1)
                 const uint32_t te = tab_u + (uint32_t)(16 * (pl + kPxLanes * (u0 + i)));
-                const int rep = lds32(te + 12u);
+                const int rep = (int)lds_u32(te + 12u);
                 const int nx = (rep & 0xff) * (rep >> 8) - 1;
                 if (nx > 0) {
-                  const uint32_t ea = sE_u + (uint32_t)lds32(te + 8u) * 128u + (uint32_t)(piece << 4);
+                  const uint32_t ea = sE_u + lds_u32(te + 8u) * 128u + (uint32_t)(piece << 4);
                   for (int x = 0; x < nx; ++x) {
                     float e8[8];
-                    unpack8(lds128(ea + 128u * (uint32_t)x), e8);
+                    unpack8(lds_v4(ea + 128u * (uint32_t)x), e8);
 #pragma unroll
                     for (int q = 0; q < 8; ++q) g[q] += e8[q];
                   }
@@ -500,14 +473,13 @@ conv3x3_gather_kernel(const __grid_constant__ CUtensorMap tmap_w, const __grid_c
                 else y[q] = cP[q] * t - fmaf(cR[q], y[q], cQ[q]);
               }
               const uint4 o = pack8(y);
-              asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};"
-                           ::"r"(dst0 + (uint32_t)(kPxLanes * 128 * (u0 + i))), "r"(o.x), "r"(o.y), "r"(o.z), "r"(o.w) : "memory");
+              sts_v4(dst0 + (uint32_t)(kPxLanes * 128 * (u0 + i)), o.x, o.y, o.z, o.w);
             }
           }
         }
       }
       // generic-proxy writes -> visible to the tensor core's (async-proxy) reads, then one arrival per producer thread
-      asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+      fence_proxy_async_smem();
       mbar_arrive(&full_a[j_as]);
       if (++j_kc == nchunks) j_kc = 0;
       if (++j_as == nA) j_as = 0;
@@ -518,11 +490,11 @@ conv3x3_gather_kernel(const __grid_constant__ CUtensorMap tmap_w, const __grid_c
       }
     }
   }
-  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+  tcgen05_before_sync();
   __syncthreads();
   if (warp == 1) {
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "n"(kTmemCols) : "memory");
+    tcgen05_after_sync();
+    tmem_dealloc<kTmemCols>(tmem_base);
   }
 }
 

@@ -19,12 +19,12 @@
 // staging tile -> TMA store (clips the ragged image edge) -> replication-count-weighted per-channel column sums of the
 // stored tile (BN batch statistics of the resampled tensor); the last CTA finalises the statistics.
 #include "conv_common.cuh"
-#include <atomic>
 #include <mutex>
 
 namespace mrfp {
 namespace {
 using namespace convk;
+using namespace ptx;
 
 constexpr int kThreads = 192;
 
@@ -67,20 +67,20 @@ conv3x3_tc_kernel(const __grid_constant__ CUtensorMap tmap_in, const __grid_cons
   const int nk = 9 * (CIN / kBlockK);       // k-steps per tile
 
   if (threadIdx.x == 0) {
-    asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(&tmap_in)) : "memory");
-    asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(&tmap_w)) : "memory");
-    asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(&tmap_out)) : "memory");
+    prefetch_tensormap(&tmap_in);
+    prefetch_tensormap(&tmap_w);
+    prefetch_tensormap(&tmap_out);
     for (int i = 0; i < C::kStages; ++i) { mbar_init(&full[i], 1); mbar_init(&empty[i], 1); }
     for (int i = 0; i < 2; ++i) { mbar_init(&tmem_full[i], 1); mbar_init(&tmem_empty[i], 4); }
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    mbar_fence_init();
   }
   if (warp == 1) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_ptr)), "n"(C::kTmemCols) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+    tmem_alloc<C::kTmemCols>(tmem_ptr);
+    tmem_relinquish();
   }
-  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+  tcgen05_before_sync();
   __syncthreads();
-  asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+  tcgen05_after_sync();
   const uint32_t tmem_base = *tmem_ptr;
   pdl_sync();                                 // set-up above overlaps the previous kernel's tail
 
@@ -106,7 +106,7 @@ conv3x3_tc_kernel(const __grid_constant__ CUtensorMap tmap_in, const __grid_cons
       }
     }
     // all loads of this CTA are in flight: let the next kernel of the stream start its set-up (PDL)
-    asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
+    pdl_trigger();
   } else if (warp == 1) {
     // ===================== MMA issuer =====================
     // The whole warp walks the loops with warp-uniform values (descriptors stay in uniform registers); one elected
@@ -120,11 +120,11 @@ conv3x3_tc_kernel(const __grid_constant__ CUtensorMap tmap_in, const __grid_cons
     for (int t = blockIdx.x; t < num_tiles; t += gridDim.x, ++it) {
       const int acc = it & 1;
       mbar_wait(&tmem_empty[acc], ((it >> 1) & 1) ^ 1);
-      asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+      tcgen05_after_sync();
       const uint32_t d_tmem = tmem_u + (uint32_t)(acc * C::kMT * COUT);
       for (int ks = 0; ks < nk; ++ks) {
         mbar_wait(&full[stage], phase);
-        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+        tcgen05_after_sync();
         if (elect_one()) {
           const uint64_t da = make_desc_sw128(sA_u + stage * C::kAStageBytes);
           const uint64_t db = make_desc_sw128(sB_u + stage * C::kBTileBytes);
@@ -149,11 +149,11 @@ conv3x3_tc_kernel(const __grid_constant__ CUtensorMap tmap_in, const __grid_cons
     conv_epilogue<COUT, T, kTileH, kTileW, C::kMT, false, 1>(es, tmem_base, tmap_out, tiles_h, tiles_w, num_tiles, cnt_h, cnt_w,
                                                                 stat_acc, rev, fin, add_src, H, W);
   }
-  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+  tcgen05_before_sync();
   __syncthreads();
   if (warp == 1) {
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "n"(C::kTmemCols) : "memory");
+    tcgen05_after_sync();
+    tmem_dealloc<C::kTmemCols>(tmem_base);
   }
 }
 
@@ -232,12 +232,7 @@ int launch(const T* in, const T* wpack, T* out, int N, int H, int W, int cin, in
   const int num_tiles = N * tiles_h * tiles_w;
   const int grid = num_tiles < di.sm_count ? num_tiles : di.sm_count;
   auto kern = conv3x3_tc_kernel<COUT, T>;
-  static std::atomic<unsigned long long> attr_done{0};           // per device, once: the opt-in shared-memory size
-  const unsigned long long bit = 1ull << (di.device & 63);
-  if (!(attr_done.load(std::memory_order_acquire) & bit)) {
-    MRFP_CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg<COUT>::kSmemBytes));
-    attr_done.fetch_or(bit, std::memory_order_release);
-  }
+  MRFP_SMEM_OPT_IN(kern, Cfg<COUT>::kSmemBytes, di.device);
   launch_k(kern, dim3(grid), dim3(kThreads), Cfg<COUT>::kSmemBytes, stream, m->in, m->w, m->out, cin, dil, tiles_h, tiles_w,
            num_tiles, cnt_h, cnt_w, stat_acc, rev, fin, add_src, H, W);
   MRFP_CUDA_TRY(cudaGetLastError());

@@ -12,7 +12,7 @@
 // Backward per stage: bn_bwd_reduce (sums over replicas) -> bn_bwd_apply (dY at conv resolution) -> dgrad conv
 // (the same conv kernel with rotated, transposed weights).  No weight gradients (deepv3.py:221-237).
 #include "hrfp.cuh"
-#include "tma.cuh"
+#include "ptx.cuh"
 #include <math.h>
 #include <stdlib.h>
 #include <string.h>
@@ -45,24 +45,8 @@ template <> struct Elem<float> {
   }
 };
 template <> struct Elem<__nv_bfloat16> {
-  static __device__ __forceinline__ void load8(const __nv_bfloat16* p, float (&v)[8]) {
-    const uint4 r = *reinterpret_cast<const uint4*>(p);
-    const uint32_t w[4] = {r.x, r.y, r.z, r.w};
-#pragma unroll
-    for (int i = 0; i < 4; ++i) {
-      v[2 * i] = __uint_as_float(w[i] << 16);
-      v[2 * i + 1] = __uint_as_float(w[i] & 0xffff0000u);
-    }
-  }
-  static __device__ __forceinline__ void store8(__nv_bfloat16* p, const float (&v)[8]) {
-    uint32_t w[4];
-#pragma unroll
-    for (int i = 0; i < 4; ++i) {
-      const __nv_bfloat162 h = __floats2bfloat162_rn(v[2 * i], v[2 * i + 1]);
-      w[i] = *reinterpret_cast<const uint32_t*>(&h);
-    }
-    *reinterpret_cast<uint4*>(p) = make_uint4(w[0], w[1], w[2], w[3]);
-  }
+  static __device__ __forceinline__ void load8(const __nv_bfloat16* p, float (&v)[8]) { unpack8(*reinterpret_cast<const uint4*>(p), v); }
+  static __device__ __forceinline__ void store8(__nv_bfloat16* p, const float (&v)[8]) { *reinterpret_cast<uint4*>(p) = pack8(v); }
   static __device__ __forceinline__ float to_float(__nv_bfloat16 x) { return __bfloat162float(x); }
   static __device__ __forceinline__ __nv_bfloat16 from_float(float x) { return __float2bfloat16_rn(x); }
   typedef uint4 Raw;
@@ -179,7 +163,7 @@ nchw_to_nhwc_stm_kernel(const float* __restrict__ src, __nv_bfloat16* __restrict
       r[2] = *reinterpret_cast<const uint32_t*>(&h2); r[3] = *reinterpret_cast<const uint32_t*>(&h3);
     }
     const int px = it * 32 + prow;
-    const uint32_t addr = tma::smem_u32(sm + px * 128 + ((warp ^ stm_swz(px)) << 4));
+    const uint32_t addr = ptx::smem_u32(sm + px * 128 + ((warp ^ stm_swz(px)) << 4));
     asm volatile("stmatrix.sync.aligned.m8n8.x4.trans.shared.b16 [%0], {%1, %2, %3, %4};"
                  ::"r"(addr), "r"(r[0]), "r"(r[1]), "r"(r[2]), "r"(r[3]) : "memory");
   }
@@ -358,15 +342,15 @@ hrfp_plus_bilinear_staged_kernel(const T* __restrict__ y, float* __restrict__ ou
   const int w_hi = min(LW - 1, (int)(rw * (float)min(w0 + kLayPx - 1, OW - 1)) + 1);
   const int cnt = min(kSegFloats, (w_hi - ws + 4) & ~3);
   if (t == 0) {
-    tma::mbar_init(&bar, 1);
-    tma::mbar_fence_init();
-    tma::mbar_expect_tx(&bar, (uint32_t)(nch * 2 * cnt) * 4u);
+    ptx::mbar_init(&bar, 1);
+    ptx::mbar_fence_init();
+    ptx::mbar_expect_tx(&bar, (uint32_t)(nch * 2 * cnt) * 4u);
   }
   __syncthreads();
   if (t < 2 * nch) {
     const int c = t >> 1, r = t & 1;
     const float* src = add_lo + (((size_t)n * C + c0 + c) * LH + h1 + (r ? h1p : 0)) * LW + ws;
-    tma::bulk_load(stage + (size_t)t * kSegFloats, src, (uint32_t)cnt * 4u, &bar);
+    ptx::bulk_load(stage + (size_t)t * kSegFloats, src, (uint32_t)cnt * 4u, &bar);
   }
   const int sh = idx_h ? idx_h[oh] : oh;
   const T* row = y + ((size_t)n * IH + sh) * IW * C;
@@ -395,7 +379,7 @@ hrfp_plus_bilinear_staged_kernel(const T* __restrict__ y, float* __restrict__ ou
     }
   }
   __syncthreads();
-  tma::mbar_wait(&bar, 0);
+  ptx::mbar_wait(&bar, 0);
   // vertical blend of the two staged rows, vb[c][k] = hl0 * r0[k] + hl1 * r1[k], written back over row 0 SPLIT BY PARITY
   // (even columns in floats [0, 36), odd columns in [36, 72)): at the x2 scale consecutive lanes read every second
   // column, which is a 2-way bank conflict on the plain layout and conflict-free on the split one
@@ -495,25 +479,25 @@ hrfp_plus_tail_ldm_kernel(const __nv_bfloat16* __restrict__ y, float* __restrict
   const int w_hi = min(LW - 1, (int)(rw * (float)w_last) + 1);
   const int cnt = min(kLdmSeg, (w_hi - ws + 4) & ~3);
   if (t == 0) {
-    tma::mbar_init(&bar, 1);
-    tma::mbar_fence_init();
-    tma::mbar_expect_tx(&bar, (uint32_t)(64 * 2 * cnt) * 4u);
+    ptx::mbar_init(&bar, 1);
+    ptx::mbar_fence_init();
+    ptx::mbar_expect_tx(&bar, (uint32_t)(64 * 2 * cnt) * 4u);
   }
   __syncthreads();
   if (t < 128) {                                                                     // the two low-resolution rows of 64 channels
     const int c = t >> 1, r = t & 1;
     const float* src = add_lo + (((size_t)n * C + c0 + c) * LH + h1 + (r ? h1p : 0)) * LW + ws;
-    tma::bulk_load(stage + (size_t)(r * 64 + c) * kLdmSeg, src, (uint32_t)cnt * 4u, &bar);
+    ptx::bulk_load(stage + (size_t)(r * 64 + c) * kLdmSeg, src, (uint32_t)cnt * 4u, &bar);
   }
   // the span of the source row this tile gathers from, 64 channels of every pixel
   const int s0 = idx_w[w0], nsp = idx_w[w_last] - s0 + 1;
   const __nv_bfloat16* yrow = y + (((size_t)n * IH + idx_h[oh]) * IW + s0) * C + c0;
   for (int e = t; e < nsp * 8; e += 256) {
     const int p = e >> 3, ch = e & 7;
-    const uint32_t dst = tma::smem_u32(ysm + p * 128 + ((ch ^ (p & 7)) << 4));
-    asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(dst), "l"(yrow + (size_t)p * C + ch * 8) : "memory");
+    const uint32_t dst = ptx::smem_u32(ysm + p * 128 + ((ch ^ (p & 7)) << 4));
+    ptx::cp_async_cg16(dst, yrow + (size_t)p * C + ch * 8);
   }
-  asm volatile("cp.async.commit_group;" ::: "memory");
+  ptx::cp_async_commit();
   if (t < 128) {
     const int ow = min(w0 + t, OW - 1);
     const float w1r = rw * (float)ow;
@@ -522,8 +506,8 @@ hrfp_plus_tail_ldm_kernel(const __nv_bfloat16* __restrict__ y, float* __restrict
     pix[t] = make_float4(__int_as_float(w1 - ws), __int_as_float(w1 - ws + (w1 < LW - 1 ? 1 : 0)), 1.f - wl1, wl1);
     spx[t] = idx_w[ow] - s0;
   }
-  asm volatile("cp.async.wait_group 0;" ::: "memory");
-  tma::mbar_wait(&bar, 0);
+  ptx::cp_async_wait<0>();
+  ptx::mbar_wait(&bar, 0);
   __syncthreads();
   {                                                                                  // vertical blend in place over row 0
     const int c = t >> 2;
@@ -545,10 +529,9 @@ hrfp_plus_tail_ldm_kernel(const __nv_bfloat16* __restrict__ y, float* __restrict
   for (int iter = 0; iter < 4; ++iter) {
     // lane L supplies row (L & 7) of matrix (L >> 3): the source pixel of destination pixel (4 iter + L/8) * 8 + L%8
     const int sidx = spx[(4 * iter + (lane >> 3)) * 8 + (lane & 7)];
-    const uint32_t addr = tma::smem_u32(ysm + sidx * 128 + ((warp ^ (sidx & 7)) << 4));
+    const uint32_t addr = ptx::smem_u32(ysm + sidx * 128 + ((warp ^ (sidx & 7)) << 4));
     uint32_t r[4];
-    asm volatile("ldmatrix.sync.aligned.m8n8.x4.trans.shared.b16 {%0, %1, %2, %3}, [%4];"
-                 : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]) : "r"(addr));
+    ptx::ldsm_x4_trans(addr, r);
 #pragma unroll
     for (int m = 0; m < 4; ++m) {
       const int px = (4 * iter + m) * 8 + 2 * (lane & 3);                            // this thread's pixel pair of matrix m
@@ -1290,12 +1273,7 @@ rankk_expand_kernel(const __nv_bfloat16* __restrict__ G, const __nv_bfloat16* __
     float g[32];
     const uint4* gp = reinterpret_cast<const uint4*>(G + px * 64);
 #pragma unroll
-    for (int q = 0; q < 4; ++q) {
-      const uint4 v = __ldg(gp + q);
-      const uint32_t w[4] = {v.x, v.y, v.z, v.w};
-#pragma unroll
-      for (int j = 0; j < 4; ++j) { g[8 * q + 2 * j] = __uint_as_float(w[j] << 16); g[8 * q + 2 * j + 1] = __uint_as_float(w[j] & 0xffff0000u); }
-    }
+    for (int q = 0; q < 4; ++q) unpack8(__ldg(gp + q), reinterpret_cast<float (&)[8]>(g[8 * q]));
     float o[8];
 #pragma unroll
     for (int j = 0; j < 8; ++j) {
@@ -1304,13 +1282,7 @@ rankk_expand_kernel(const __nv_bfloat16* __restrict__ G, const __nv_bfloat16* __
       for (int k = 0; k < 32; ++k) a = fmaf(g[k], s_w[(c0 + j) * 32 + k], a);
       o[j] = a;
     }
-    uint32_t pk[4];
-#pragma unroll
-    for (int j = 0; j < 4; ++j) {
-      const __nv_bfloat162 h2 = __floats2bfloat162_rn(o[2 * j], o[2 * j + 1]);
-      pk[j] = *reinterpret_cast<const uint32_t*>(&h2);
-    }
-    *reinterpret_cast<uint4*>(dA + px * C + c0) = make_uint4(pk[0], pk[1], pk[2], pk[3]);
+    *reinterpret_cast<uint4*>(dA + px * C + c0) = pack8(o);
   }
 }
 

@@ -12,7 +12,7 @@
 // Statistics are two-pass over the resident copy (mean first, then centred squares; double across lanes) — the same
 // biased variance F.instance_norm uses.  Planes too large for an 8-CTA cluster fall back to re-reading global memory.
 #include "hrfp.cuh"
-#include "tma.cuh"
+#include "ptx.cuh"
 #include <cooperative_groups.h>
 #include <math.h>
 #include <atomic>
@@ -70,8 +70,8 @@ __device__ __forceinline__ void issue_slice_load(float* dst, const float* src, i
       const int nchunk = (len + kChunkElems - 1) / kChunkElems;
       for (int k = 0; k < nchunk; ++k) {
         const int n = min(kChunkElems, len - k * kChunkElems);
-        tma::mbar_expect_tx(&bars[k], (uint32_t)n * 4u);
-        tma::bulk_load(dst + k * kChunkElems, src + k * kChunkElems, (uint32_t)n * 4u, &bars[k]);
+        ptx::mbar_expect_tx(&bars[k], (uint32_t)n * 4u);
+        ptx::bulk_load(dst + k * kChunkElems, src + k * kChunkElems, (uint32_t)n * 4u, &bars[k]);
       }
     }
   } else {
@@ -97,9 +97,9 @@ instnorm_fwd_kernel(const float* __restrict__ x, const float* __restrict__ gamma
   __shared__ __align__(8) uint64_t ps_bar;           // rank 0: the plane-sum partials land here (st.async + complete_tx)
   if (cs > 1) {
     if (psum && cr == 0 && threadIdx.x == 0) {
-      tma::mbar_init(&ps_bar, 1);
-      tma::mbar_fence_init();
-      tma::mbar_expect_tx(&ps_bar, cs * 8u);
+      ptx::mbar_init(&ps_bar, 1);
+      ptx::mbar_fence_init();
+      ptx::mbar_expect_tx(&ps_bar, cs * 8u);
     }
     cl_arrive();                                   // matched by the cl_wait() in front of the first push
   }
@@ -114,8 +114,8 @@ instnorm_fwd_kernel(const float* __restrict__ x, const float* __restrict__ gamma
   if (RESIDENT) {
     if (VEC) {
       if (tid == 0) {
-        for (int k = 0; k < nchunk; ++k) tma::mbar_init(&bars[k], 1);
-        tma::mbar_fence_init();
+        for (int k = 0; k < nchunk; ++k) ptx::mbar_init(&bars[k], 1);
+        ptx::mbar_fence_init();
       }
       __syncthreads();
     }
@@ -128,7 +128,7 @@ instnorm_fwd_kernel(const float* __restrict__ x, const float* __restrict__ gamma
   float acc = 0.f;
   if (VEC) {
     for (int k = 0; k < nchunk; ++k) {
-      if (RESIDENT) tma::mbar_wait(&bars[k], 0);
+      if (RESIDENT) ptx::mbar_wait(&bars[k], 0);
       const int n4 = min(kChunkElems, len - k * kChunkElems) >> 2;
       const float4* p = reinterpret_cast<const float4*>(in + k * kChunkElems);
       float4 a4 = make_float4(0.f, 0.f, 0.f, 0.f);
@@ -212,12 +212,12 @@ instnorm_fwd_kernel(const float* __restrict__ x, const float* __restrict__ gamma
       // store that completes bytes on rank 0's mbarrier carries the value without any fence; the other CTAs are done.
       if (tid == 0) {
         uint32_t dst, bar;
-        asm volatile("mapa.shared::cluster.u32 %0, %1, 0;" : "=r"(dst) : "r"(tma::smem_u32(&s_ps[cr])));
-        asm volatile("mapa.shared::cluster.u32 %0, %1, 0;" : "=r"(bar) : "r"(tma::smem_u32(&ps_bar)));
+        asm volatile("mapa.shared::cluster.u32 %0, %1, 0;" : "=r"(dst) : "r"(ptx::smem_u32(&s_ps[cr])));
+        asm volatile("mapa.shared::cluster.u32 %0, %1, 0;" : "=r"(bar) : "r"(ptx::smem_u32(&ps_bar)));
         asm volatile("st.async.weak.shared::cluster.mbarrier::complete_tx::bytes.b64 [%0], %1, [%2];"
                      ::"r"(dst), "l"(__double_as_longlong(ys)), "r"(bar) : "memory");
         if (cr == 0) {
-          tma::mbar_wait(&ps_bar, 0);
+          ptx::mbar_wait(&ps_bar, 0);
           double t = 0.0;
           for (unsigned k = 0; k < cs; ++k) t += s_ps[k];
           psum[plane] = t;
@@ -261,17 +261,17 @@ instnorm_bwd_kernel(const float* __restrict__ gy, const float* __restrict__ x, c
   if (RESIDENT) {
     if (VEC) {
       if (tid == 0) {
-        for (int k = 0; k < 2 * nchunk; ++k) tma::mbar_init(&bars[k], 1);
-        tma::mbar_fence_init();
+        for (int k = 0; k < 2 * nchunk; ++k) ptx::mbar_init(&bars[k], 1);
+        ptx::mbar_fence_init();
       }
       __syncthreads();
       if (tid == 0) {                               // interleave the two streams chunk by chunk
         for (int k = 0; k < nchunk; ++k) {
           const uint32_t nb = (uint32_t)min(kChunkElems, len - k * kChunkElems) * 4u;
-          tma::mbar_expect_tx(&bars[2 * k], nb);
-          tma::bulk_load(bx + k * kChunkElems, x + off + k * kChunkElems, nb, &bars[2 * k]);
-          tma::mbar_expect_tx(&bars[2 * k + 1], nb);
-          tma::bulk_load(bg + k * kChunkElems, gy + off + k * kChunkElems, nb, &bars[2 * k + 1]);
+          ptx::mbar_expect_tx(&bars[2 * k], nb);
+          ptx::bulk_load(bx + k * kChunkElems, x + off + k * kChunkElems, nb, &bars[2 * k]);
+          ptx::mbar_expect_tx(&bars[2 * k + 1], nb);
+          ptx::bulk_load(bg + k * kChunkElems, gy + off + k * kChunkElems, nb, &bars[2 * k + 1]);
         }
       }
     } else {
@@ -298,7 +298,7 @@ instnorm_bwd_kernel(const float* __restrict__ gy, const float* __restrict__ x, c
   };
   if (VEC) {
     for (int k = 0; k < nchunk; ++k) {
-      if (RESIDENT) { tma::mbar_wait(&bars[2 * k], 0); tma::mbar_wait(&bars[2 * k + 1], 0); }
+      if (RESIDENT) { ptx::mbar_wait(&bars[2 * k], 0); ptx::mbar_wait(&bars[2 * k + 1], 0); }
       const int n4 = min(kChunkElems, len - k * kChunkElems) >> 2;
       const float4* p = reinterpret_cast<const float4*>(px + k * kChunkElems);
       const float4* q = reinterpret_cast<const float4*>(pg + k * kChunkElems);
@@ -458,8 +458,8 @@ instnorm_ring_kernel(const RingArgs a) {
   const int nsync = cs == 1 ? 0 : (BWD ? 1 : 2);                    // cluster barriers before the output pass
 
   if (tid == 0) {
-    for (int s = 0; s < kRSlots; ++s) { tma::mbar_init(&full[s], 1); tma::mbar_init(&empty[s], kRWarps); }
-    tma::mbar_fence_init();
+    for (int s = 0; s < kRSlots; ++s) { ptx::mbar_init(&full[s], 1); ptx::mbar_init(&empty[s], kRWarps); }
+    ptx::mbar_fence_init();
   }
   __syncthreads();
 
@@ -468,12 +468,12 @@ instnorm_ring_kernel(const RingArgs a) {
     auto issue = [&](int plane, int j0, int j1) {                   // fills j0..j1-1 of `plane` (lane 0 only)
       for (int j = j0; j < j1; ++j, ++fill) {
         const int slot = fill % kRSlots, round = fill / kRSlots;
-        if (round > 0) tma::mbar_wait(&empty[slot], (round - 1) & 1);
+        if (round > 0) ptx::mbar_wait(&empty[slot], (round - 1) & 1);
         const int chunk = BWD ? (j >> 1) : j;
         const float* base = (BWD && (j & 1)) ? a.gy : a.x;
         const uint32_t bytes = (uint32_t)min(kRChunk, len - chunk * kRChunk) * 4u;
-        tma::mbar_expect_tx(&full[slot], bytes);
-        tma::bulk_load(ring + (size_t)slot * kRChunk, base + (long long)plane * a.HW + begin + chunk * kRChunk, bytes, &full[slot]);
+        ptx::mbar_expect_tx(&full[slot], bytes);
+        ptx::bulk_load(ring + (size_t)slot * kRChunk, base + (long long)plane * a.HW + begin + chunk * kRChunk, bytes, &full[slot]);
       }
     };
     if (lane == 0 && q < a.planes) issue(q, 0, F);
@@ -493,10 +493,10 @@ instnorm_ring_kernel(const RingArgs a) {
       const float gm = a.gamma ? a.gamma[c] : 1.f, bt = a.beta ? a.beta[c] : 0.f;
       const long long off = (long long)p * a.HW + begin;
       auto slot_of = [&](int j) { return (cfill + j) % kRSlots; };
-      auto wait_fill = [&](int j) { tma::mbar_wait(&full[slot_of(j)], ((cfill + j) / kRSlots) & 1); };
+      auto wait_fill = [&](int j) { ptx::mbar_wait(&full[slot_of(j)], ((cfill + j) / kRSlots) & 1); };
       auto release = [&](int j) {                                   // this warp is done with fill j of the plane
         __syncwarp();
-        if (lane == 0) tma::mbar_arrive(&empty[slot_of(j)]);
+        if (lane == 0) ptx::mbar_arrive(&empty[slot_of(j)]);
       };
       if (!BWD) {
         // pass 1: sum -> mean (chunk by chunk as the copies land)
@@ -582,7 +582,7 @@ instnorm_ring_kernel(const RingArgs a) {
                                 sc * (gp.w - m1 - xh.w * m2));
           }
           // the slots were written through the generic proxy: order those writes before the bulk copy that refills them
-          asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+          ptx::fence_proxy_async_smem();
           release(2 * j); release(2 * j + 1);
         }
         if (cr == 0 && tid == 0) { a.dgamma_part[p] = (float)t.b; a.dbeta_part[p] = (float)t.a; }

@@ -21,6 +21,7 @@
 // A register-staged variant of the same algorithm (no TMA; scalar loads) handles planes whose size or base
 // address is not a multiple of 16 bytes.
 #include "common.cuh"
+#include "ptx.cuh"
 #include <cooperative_groups.h>
 #include <math.h>
 #include <stdlib.h>
@@ -30,6 +31,7 @@ namespace cg = cooperative_groups;
 
 namespace mrfp {
 namespace {
+using namespace ptx;
 
 constexpr int kConsumers = 512;                 // consumer threads (16 warps)
 constexpr int kWarps = kConsumers / 32;
@@ -237,34 +239,6 @@ __device__ __forceinline__ float2 np_plane_coef(int p, bool publish, const doubl
 }
 
 // ------------------------------------------------------------------------------------------------------
-// mbarrier / bulk-copy primitives
-// ------------------------------------------------------------------------------------------------------
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(uint64_t* bar, uint32_t count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count));
-}
-__device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
-  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ void mbar_expect_tx(uint64_t* bar, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "WAIT_%=:\n\t"
-      "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n\t"
-      "@p bra DONE_%=;\n\t"
-      "bra WAIT_%=;\n\t"
-      "DONE_%=:\n\t}" ::"r"(smem_u32(bar)), "r"(parity) : "memory");
-}
-__device__ __forceinline__ void bulk_load(void* smem_dst, const void* gsrc, uint32_t bytes, uint64_t* bar,
-                                          uint64_t policy) {
-  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes.L2::cache_hint [%0], [%1], %2, [%3], %4;"
-               ::"r"(smem_u32(smem_dst)), "l"(gsrc), "r"(bytes), "r"(smem_u32(bar)), "l"(policy) : "memory");
-}
-
-// ------------------------------------------------------------------------------------------------------
 // TMA-ring kernel with grid-wide dynamic unit queues (planes and base addresses 16-byte aligned)
 // ------------------------------------------------------------------------------------------------------
 // SMs do not stream from HBM at the same rate (the slowest took 40 % longer than the fastest on a static
@@ -303,7 +277,7 @@ __device__ __forceinline__ void tmem_fetch(uint32_t taddr, float4 (&v)[kBatch]) 
       : "=f"(v[0].x), "=f"(v[0].y), "=f"(v[0].z), "=f"(v[0].w), "=f"(v[1].x), "=f"(v[1].y), "=f"(v[1].z), "=f"(v[1].w),
         "=f"(v[2].x), "=f"(v[2].y), "=f"(v[2].z), "=f"(v[2].w), "=f"(v[3].x), "=f"(v[3].y), "=f"(v[3].z), "=f"(v[3].w)
       : "r"(taddr));
-  asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+  tcgen05_wait_ld();
 }
 
 template <bool BWD>
@@ -352,16 +326,16 @@ npplus_ring_kernel(const float* __restrict__ x, const float* __restrict__ alpha,
 
   if (tid == 0) {
     for (int s = 0; s < S; ++s) { mbar_init(&full[s], 1); mbar_init(&empty[s], kWarps); slot_cnt[s] = 0; }
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    mbar_fence_init();
     if (blockIdx.x == 0) ctrl->counter_b = 0;            // read behind the second grid barrier only
   }
   if (is_producer && T > RG) {                           // the whole TMEM (one CTA per SM, no MMA in this kernel)
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], 512;" ::"r"(smem_u32(&tmem_base_s)) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+    tmem_alloc<512>(&tmem_base_s);
+    tmem_relinquish();
+    tcgen05_before_sync();
   }
   __syncthreads();
-  asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+  tcgen05_after_sync();
   // this thread's window into TMEM: its own lane, 16 columns per parked unit
   const uint32_t tmem_mine = T > RG ? tmem_base_s + ((uint32_t)((warp & 3) * 32) << 16) + (uint32_t)((warp >> 2) * 16) : 0u;
 
@@ -377,17 +351,14 @@ npplus_ring_kernel(const float* __restrict__ x, const float* __restrict__ alpha,
   // ---------------- phase A ----------------
   if (is_producer) {
     if (lane == 0) {
-      uint64_t pol_keep, pol_mid, pol_stream;
-      asm volatile("createpolicy.fractional.L2::evict_last.b64 %0, 1.0;" : "=l"(pol_keep));
-      asm volatile("createpolicy.fractional.L2::evict_normal.b64 %0, 1.0;" : "=l"(pol_mid));
-      asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(pol_stream));
+      const uint64_t pol_keep = policy_evict_last(), pol_mid = policy_evict_normal(), pol_stream = policy_evict_first();
       auto issue = [&](int u, uint64_t pol) {
         if (k > 0) mbar_wait(&empty[s], (k - 1) & 1);    // all 16 warps released the previous fill of this slot
         uint32_t bytes;
         const long long off = unit_src(u, &bytes);
         slot_unit[s] = u;
         mbar_expect_tx(&full[s], bytes);
-        bulk_load(ring + (size_t)s * kUnitVecs, xv + off, bytes, &full[s], pol);
+        bulk_load_hint(ring + (size_t)s * kUnitVecs, xv + off, bytes, &full[s], pol);
         advance();
       };
       for (int j = 0; j < T; ++j) issue(head0 + j, pol_stream);
@@ -482,8 +453,7 @@ npplus_ring_kernel(const float* __restrict__ x, const float* __restrict__ alpha,
 
   // ---------------- phase B ----------------
   if (is_producer) {
-    uint64_t pol_stream;
-    asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(pol_stream));
+    const uint64_t pol_stream = policy_evict_first();
     // software pipeline, one batch deep: while batch j is being issued (which blocks on free slots), the index of
     // batch j+1 and the inputs of its (a, b) pairs are already in flight
     auto grab = [&]() {
@@ -523,7 +493,7 @@ npplus_ring_kernel(const float* __restrict__ x, const float* __restrict__ alpha,
           slot_unit[s] = uq;
           slot_coef[s] = make_float2(ax, ay);
           mbar_expect_tx(&full[s], bytes);
-          bulk_load(ring + (size_t)s * kUnitVecs, xv + off, bytes, &full[s], pol_stream);
+          bulk_load_hint(ring + (size_t)s * kUnitVecs, xv + off, bytes, &full[s], pol_stream);
         }
         advance();
       }
@@ -574,11 +544,11 @@ npplus_ring_kernel(const float* __restrict__ x, const float* __restrict__ alpha,
     if (g.heads_last) emit_heads();
   }
   if (T > RG) {
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+    tcgen05_before_sync();
     __syncthreads();
     if (is_producer) {
-      asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-      asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, 512;" ::"r"(tmem_base_s) : "memory");
+      tcgen05_after_sync();
+      tmem_dealloc<512>(tmem_base_s);
     }
   }
   if (trace) { __syncthreads(); stamp(4); }

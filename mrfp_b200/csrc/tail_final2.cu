@@ -37,13 +37,13 @@
 // cycles per 64-pixel tile, a lane-indexed register pick compiles to divergent branches, a proxy fence per issue and
 // global index look-ups sit on the critical path of every barrier.  This form: 133 / 210 us.
 #include "hrfp.cuh"
-#include "tma.cuh"
+#include "ptx.cuh"
 #include <mutex>
 
 namespace mrfp {
 namespace {
 
-using namespace tma;
+using namespace ptx;
 
 constexpr int kC = 256;              // channels of OCout_dec (widths[3])
 constexpr int kCls = 24;             // classes, padded to three n-blocks of 8 (forward) / 32 (backward k-blocks)
@@ -56,19 +56,11 @@ __device__ __forceinline__ void ldsm_x4(uint32_t addr, uint32_t (&r)[4]) {
 __device__ __forceinline__ void ldsm_x2(uint32_t addr, uint32_t (&r)[2]) {
   asm volatile("ldmatrix.sync.aligned.m8n8.x2.shared.b16 {%0, %1}, [%2];" : "=r"(r[0]), "=r"(r[1]) : "r"(addr));
 }
-__device__ __forceinline__ void ldsm_x4_t(uint32_t addr, uint32_t (&r)[4]) {
-  asm volatile("ldmatrix.sync.aligned.m8n8.x4.trans.shared.b16 {%0, %1, %2, %3}, [%4];"
-               : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]) : "r"(addr));
-}
 // D += A (16x16, row) * B (16x8, col), bf16 operands, fp32 accumulators
 __device__ __forceinline__ void mma_bf16(float (&d)[4], const uint32_t (&a)[4], uint32_t b0, uint32_t b1) {
   asm volatile("mma.sync.aligned.m16n8k16.row.col.f32.bf16.bf16.f32 {%0, %1, %2, %3}, {%4, %5, %6, %7}, {%8, %9}, {%0, %1, %2, %3};"
                : "+f"(d[0]), "+f"(d[1]), "+f"(d[2]), "+f"(d[3])
                : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b0), "r"(b1));
-}
-__device__ __forceinline__ uint32_t pack_bf16(float lo, float hi) {
-  const __nv_bfloat162 h = __floats2bfloat162_rn(lo, hi);
-  return *reinterpret_cast<const uint32_t*>(&h);
 }
 // launch-constant arguments of both kernels
 struct TailArgs {
@@ -162,8 +154,8 @@ tail_final2_fwd_kernel(const __grid_constant__ CUtensorMap tm_y, const __grid_co
   const int q = warp & 3, u = warp >> 2;
   if (t == 0) {
     mbar_init(&bar[0], 1); mbar_init(&bar[1], 1); mbar_fence_init();
-    asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(&tm_y)) : "memory");
-    asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(&tm_lo)) : "memory");
+    prefetch_tensormap(&tm_y);
+    prefetch_tensormap(&tm_lo);
   }
   pdl_sync();
   // classifier weights -> bf16 [class][channel] (swizzled rows) in the span buffer, from there into B fragments
@@ -193,7 +185,7 @@ tail_final2_fwd_kernel(const __grid_constant__ CUtensorMap tm_y, const __grid_co
       sq[kk][2] = pack_f32x2(a.scale[c0 + 8], a.scale[c0 + 9]); sq[kk][3] = pack_f32x2(a.shift[c0 + 8], a.shift[c0 + 9]);
     }
   }
-  asm volatile("fence.proxy.async.shared::cta;" ::: "memory");   // the staging writes precede the TMA writes of buffer 0
+  fence_proxy_async_smem();   // the staging writes precede the TMA writes of buffer 0
   __syncthreads();                                     // the staging region becomes span buffer 0
   const float rh = a.OH > 1 ? (float)(LH - 1) / (float)(a.OH - 1) : 0.f;               // ATen upsample_bilinear2d(align_corners=True)
   const float rw = a.OW > 1 ? (float)(LW - 1) / (float)(a.OW - 1) : 0.f;
@@ -331,8 +323,8 @@ tail_final2_bwd_kernel(const __grid_constant__ CUtensorMap tm_y, const __grid_co
   const int amat = lane >> 3, arow = (amat & 1) * 8 + (lane & 7), akc = amat >> 1;
   if (t == 0) {
     mbar_init(&bar[0], 1); mbar_init(&bar[1], 1); mbar_fence_init();
-    asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(&tm_y)) : "memory");
-    if (g_tma) asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(&tm_g)) : "memory");
+    prefetch_tensormap(&tm_y);
+    if (g_tma) prefetch_tensormap(&tm_g);
   }
   pdl_sync();
   // W2^T -> bf16 [channel][class] (16-byte chunks swizzled by (channel >> 1) & 3) in the span buffer, then into B fragments
@@ -376,7 +368,7 @@ tail_final2_bwd_kernel(const __grid_constant__ CUtensorMap tm_y, const __grid_co
 #pragma unroll
       for (int r = 0; r < 4; ++r) wacc[i][j][r] = 0.f;
   float sg[4] = {0.f, 0.f, 0.f, 0.f};                   // bias-gradient partials of classes warp + 8 i (this lane's two pixels)
-  asm volatile("fence.proxy.async.shared::cta;" ::: "memory");   // staging writes and the zero fill precede the TMA writes
+  fence_proxy_async_smem();   // staging writes and the zero fill precede the TMA writes
   __syncthreads();                                      // the staging region becomes span buffer 0
 
   // one thread: the tile's span of Y_3 (one box: 64 px x 4 groups of 64 channels) and its [K][64] box of g (pixels beyond the row end arrive as zeros)
@@ -420,7 +412,7 @@ tail_final2_bwd_kernel(const __grid_constant__ CUtensorMap tm_y, const __grid_co
       for (int i = 0; i < 4; ++i) {                    // g tile -> bf16 [class][pixel]: a warp writes one whole 128-byte row
         const int k = warp + 8 * i;
         const float2 v = *reinterpret_cast<const float2*>(gb + k * kPx + 2 * lane);
-        *reinterpret_cast<uint32_t*>(gC + k * 128 + (((lane >> 2) ^ (k & 7)) << 4) + (lane & 3) * 4) = pack_bf16(v.x, v.y);
+        *reinterpret_cast<uint32_t*>(gC + k * 128 + (((lane >> 2) ^ (k & 7)) << 4) + (lane & 3) * 4) = pack_bf16x2(v.x, v.y);
         sg[i] += v.x + v.y;
       }
     }
@@ -436,7 +428,7 @@ tail_final2_bwd_kernel(const __grid_constant__ CUtensorMap tm_y, const __grid_co
         uint32_t pk[8] = {0u, 0u, 0u, 0u, 0u, 0u, 0u, 0u};
         if (quarter < 2) {
 #pragma unroll
-          for (int j = 0; j < 8; ++j) pk[j] = pack_bf16(gb[(16 * quarter + 2 * j) * kPx + px], gb[(16 * quarter + 2 * j + 1) * kPx + px]);
+          for (int j = 0; j < 8; ++j) pk[j] = pack_bf16x2(gb[(16 * quarter + 2 * j) * kPx + px], gb[(16 * quarter + 2 * j + 1) * kPx + px]);
         }
         uint4* dst = reinterpret_cast<uint4*>(g64 + (((size_t)c.n * a.OH + c.oh) * a.OW + c.w0 + px) * 64 + 16 * quarter);
         dst[0] = make_uint4(pk[0], pk[1], pk[2], pk[3]);
@@ -450,7 +442,7 @@ tail_final2_bwd_kernel(const __grid_constant__ CUtensorMap tm_y, const __grid_co
 #pragma unroll
         for (int kb = 0; kb < 2; ++kb) {                 // matrices: (px 0-7 | px 8-15) x (classes 16 kb + 0-7 | + 8-15)
           const int cls = 16 * kb + (amat >> 1) * 8 + (lane & 7), chunk = 2 * mt + (amat & 1);
-          ldsm_x4_t(smem_u32(gC + cls * 128 + ((chunk ^ (cls & 7)) << 4)), af[kb]);
+          ldsm_x4_trans(smem_u32(gC + cls * 128 + ((chunk ^ (cls & 7)) << 4)), af[kb]);
         }
         float acc[4][4];
 #pragma unroll
@@ -466,7 +458,7 @@ tail_final2_bwd_kernel(const __grid_constant__ CUtensorMap tm_y, const __grid_co
           }
         uint32_t r0[4], r1[4];
 #pragma unroll
-        for (int j = 0; j < 4; ++j) { r0[j] = pack_bf16(acc[j][0], acc[j][1]); r1[j] = pack_bf16(acc[j][2], acc[j][3]); }
+        for (int j = 0; j < 4; ++j) { r0[j] = pack_bf16x2(acc[j][0], acc[j][1]); r1[j] = pack_bf16x2(acc[j][2], acc[j][3]); }
         const uint4 o0 = quad_transpose(r0, tq), o1 = quad_transpose(r1, tq);     // channels 32 warp + 8 tq + 0..7
         const int p0 = 16 * mt + g8, p1 = p0 + 8;
         __nv_bfloat16* drow = dA + (((size_t)c.n * a.OH + c.oh) * a.OW + c.w0) * kC + 32 * warp + 8 * tq;
@@ -491,7 +483,7 @@ tail_final2_bwd_kernel(const __grid_constant__ CUtensorMap tm_y, const __grid_co
         for (int jp = 0; jp < 2; ++jp) {               // n-block pairs: channels 32 warp + 16 jp + {0..7, 8..15}
           const int chunk = 4 * warp + 2 * jp + bnb;   // 16-byte chunk (8 channels) of the pixel's 256 channels
           uint32_t bf[4];
-          ldsm_x4_t(span_addr(ybase, sidx, chunk), bf);
+          ldsm_x4_trans(span_addr(ybase, sidx, chunk), bf);
           bf[0] = bn_relu_x2(bf[0], sc[2 * jp][0], sc[2 * jp][1]); bf[1] = bn_relu_x2(bf[1], sc[2 * jp][0], sc[2 * jp][1]);
           bf[2] = bn_relu_x2(bf[2], sc[2 * jp + 1][0], sc[2 * jp + 1][1]); bf[3] = bn_relu_x2(bf[3], sc[2 * jp + 1][0], sc[2 * jp + 1][1]);
           mma_bf16(wacc[0][2 * jp], a0, bf[0], bf[1]);
