@@ -128,33 +128,36 @@ int    mrfp_hrfp_plan_set_fusion(mrfp_hrfp_plan_t* plan, int bits);
  *   ocout      (N,cin,xh,xw)      = OCout (+ x_add when x_add != NULL: deepv3.py:330)
  *   ocout_dec  (N,widths[3],h/2,w/2) = OCout_dec, or NULL when HRFP+ is off
  * ocout == NULL runs the encoder half only (decoder output unused when p >= 0.5); with ocout_dec == NULL as
- * well the call only leaves the state for a later mrfp_hrfp_plus_add / mrfp_hrfp_bwd in `saved`. */
-int mrfp_hrfp_fwd(const mrfp_hrfp_plan_t* plan, const float* xp,
-                  const float* const* W, const float* const* gamma, const float* const* beta,
-                  float* const* running_mean, float* const* running_var, float momentum, float eps,
-                  const float* x_add, float* ocout, float* ocout_dec,
-                  const void* lut, void* saved, void* ws, void* stream);
-
-/* Input gradient wrt xp.  g_ocout / g_ocout_dec may be NULL (that output unused). */
-int mrfp_hrfp_bwd(const mrfp_hrfp_plan_t* plan, const float* g_ocout, const float* g_ocout_dec,
-                  const float* const* gamma, const void* lut, const void* saved,
-                  float* g_xp, void* ws, void* stream);
-
-/* NP+ call 1 folded into the chain (SURVEY.md 8f-1):  ocout = OCout + NP+(xp)  — deepv3.py:316-318 followed by
+ * well the call only leaves the state for a later mrfp_hrfp_plus_add / mrfp_hrfp_bwd in `saved`.
+ * NP+ call 1 folded into the chain (SURVEY.md 8f-1):  ocout = OCout + NP+(xp)  — deepv3.py:316-318 followed by
  * :320-330 when both gates are on — without materialising NP+(xp): the plane totals of xp are taken by the layout pass
  * that feeds the chain, the per-plane (a, b) by one block, and the chain's output pass adds a*xp + b.
  *   np_alpha, np_eps (N,cin): the two Gaussian draws of deepv3.py:274-275;  np_mean (N,cin) out: plane means, needed
  *   by the backward;  np_beta (N,cin) out, may be NULL;  np_ws: >= mrfp_hrfp_np_ws_bytes(N,cin) bytes, 16-byte aligned.
- * Everything else as in mrfp_hrfp_fwd / mrfp_hrfp_bwd; g_xp receives the sum of both gradient paths into xp. */
+ * np_alpha, np_eps, np_mean and np_ws are all NULL (NP+ not folded in) or all set; folding needs ocout and no x_add. */
 size_t mrfp_hrfp_np_ws_bytes(int N, int C);
-int mrfp_hrfp_fwd_np(const mrfp_hrfp_plan_t* plan, const float* xp,
-                     const float* const* W, const float* const* gamma, const float* const* beta,
-                     float* const* running_mean, float* const* running_var, float momentum, float eps,
-                     const float* np_alpha, const float* np_eps, float* np_mean, float* np_beta, void* np_ws,
-                     float* ocout, float* ocout_dec, const void* lut, void* saved, void* ws, void* stream);
-int mrfp_hrfp_bwd_np(const mrfp_hrfp_plan_t* plan, const float* g_ocout, const float* g_ocout_dec,
-                     const float* const* gamma, const float* np_alpha, const float* np_eps, const float* np_mean,
-                     void* np_ws, const void* lut, const void* saved, float* g_xp, void* ws, void* stream);
+int mrfp_hrfp_fwd(const mrfp_hrfp_plan_t* plan, const float* xp,
+                  const float* const* W, const float* const* gamma, const float* const* beta,
+                  float* const* running_mean, float* const* running_var, float momentum, float eps,
+                  const float* x_add, const float* np_alpha, const float* np_eps, float* np_mean, float* np_beta,
+                  void* np_ws, float* ocout, float* ocout_dec, const void* lut, void* saved, void* ws, void* stream);
+
+/* The form in which the gradient of OCout_dec reaches mrfp_hrfp_bwd (`dec_form`, `g_dec`, `w2t64`). */
+#define MRFP_DEC_GRAD_NONE    0  /* OCout_dec unused: g_dec and w2t64 NULL                                   */
+#define MRFP_DEC_GRAD_F32     1  /* g_dec (N, widths[3], h/2, w/2) fp32 NCHW                                  */
+#define MRFP_DEC_GRAD_NHWC    2  /* g_dec (N, h/2, w/2, widths[3]) in the chain's element type (TF32/BF16)    */
+#define MRFP_DEC_GRAD_RANK_K  3  /* g_dec = g64 (N, h/2, w/2, 64) bf16, w2t64 (256, 64) bf16 (BF16, widths[3]==256) */
+
+/* Input gradient wrt xp.  g_ocout may be NULL (that output unused).  The NHWC and rank-K forms must be 16-byte aligned.
+ * The rank-K form is W2^T g of the classifier tail left as its two factors (mrfp_hrfp_tail_final2_bwd_rk): the stage-4
+ * dgrad accumulates g64 . w2t64^T as one more k-block on the tensor cores (fp32, one rounding together with the
+ * convolution's own sum), so the (N, h/2, w/2, 256) tensor — 604 MB at batch 8, 768^2 — is neither written nor read; when
+ * the stage-4 dgrad does not run as the operand-fused kernel, or the backward is encoder-only, the library expands the
+ * product itself.  np_*: the forward's NP+ draws, plane means and workspace when NP+ was folded in, else all NULL;
+ * g_xp then receives the sum of both gradient paths into xp (NP+ is ignored when g_ocout is NULL). */
+int mrfp_hrfp_bwd(const mrfp_hrfp_plan_t* plan, const float* g_ocout, int dec_form, const void* g_dec, const void* w2t64,
+                  const float* const* gamma, const float* np_alpha, const float* np_eps, const float* np_mean,
+                  void* np_ws, const void* lut, const void* saved, float* g_xp, void* ws, void* stream);
 
 /* HRFP+ skip add, deepv3.py:357, fused with the production of OCout_dec: out = dec1_up + OCout_dec where
  * OCout_dec = ReLU(BN(resample(conv4))) is recomputed from the state `saved` by the preceding mrfp_hrfp_fwd
@@ -176,7 +179,7 @@ int mrfp_hrfp_plus_add_bilinear(const mrfp_hrfp_plan_t* plan, const void* saved,
  *        yields the gradient to dec1 and the low-resolution half of the gradient to W2);
  *   w2 (K, 256), b2 (K) fp32;  out (N, K, h/2, w/2) fp32 NCHW.
  * Neither OCout_dec, the up-sampled dec1 nor their sum (N, 256, h/2, w/2) is materialised.
- * Backward, given g = dL/d out: g_dec_nhwc (N, h/2, w/2, 256) bf16 = W2^T g (feed it to mrfp_hrfp_bwd_nhwc),
+ * Backward, given g = dL/d out: g_dec_nhwc (N, h/2, w/2, 256) bf16 = W2^T g (mrfp_hrfp_bwd's MRFP_DEC_GRAD_NHWC),
  * g_w2 (K, 256) = sum_pixels g . OCout_dec^T (the high-resolution half of the weight gradient), g_b2 (K) = sum g; the
  * gradient to t_lo is mrfp_bilinear_up_bwd_f32(g).  MRFP_ERR_UNSUPPORTED: use mrfp_hrfp_plus_add_bilinear + a conv.
  * Inputs arrive through TMA tensor maps the plan caches per direction (re-encoded when an address or shape changes): t_lo
@@ -186,23 +189,12 @@ int mrfp_hrfp_tail_final2_fwd(const mrfp_hrfp_plan_t* plan, const void* saved, c
                               int lh, int lw, const float* w2, const float* b2, int K, float* out, void* stream);
 int mrfp_hrfp_tail_final2_bwd(const mrfp_hrfp_plan_t* plan, const void* saved, const void* lut, const float* g,
                               const float* w2, int K, void* g_dec_nhwc, float* g_w2, float* g_b2, void* stream);
-/* mrfp_hrfp_bwd / mrfp_hrfp_bwd_np with the gradient of OCout_dec in the chain's own layout (np_* all NULL: no folded NP+). */
-int mrfp_hrfp_bwd_nhwc(const mrfp_hrfp_plan_t* plan, const float* g_ocout, const void* g_dec_nhwc,
-                       const float* const* gamma, const float* np_alpha, const float* np_eps, const float* np_mean,
-                       void* np_ws, const void* lut, const void* saved, float* g_xp, void* ws, void* stream);
-
-/* The RANK-K form of the same pair (the default of the Python host): the gradient of OCout_dec is W2^T g with K <= 24
- * classes, so instead of leaving it as an (N, h/2, w/2, 256) tensor the tail's backward leaves its two factors —
- *   g64 (N, h/2, w/2, 64) bf16: g per pixel, classes beyond K zero;   w2t64 (256, 64) bf16: W2 transposed, zero-padded —
- * and mrfp_hrfp_bwd_rk lets the stage-4 dgrad accumulate g64 . w2t64^T as one more k-block on the tensor cores (fp32, one
- * rounding together with the convolution's own sum).  The 604 MB tensor (batch 8, 768^2) is neither written nor read; when
- * the stage-4 dgrad does not run as the operand-fused kernel, or the backward is encoder-only, the library expands the
- * product itself.  Everything else as mrfp_hrfp_tail_final2_bwd / mrfp_hrfp_bwd_nhwc. */
+/* The rank-K form of the same gradient (the default of the Python host; mrfp_hrfp_bwd's MRFP_DEC_GRAD_RANK_K): W2^T g
+ * with K <= 24 classes left as its two factors instead of an (N, h/2, w/2, 256) tensor —
+ *   g64 (N, h/2, w/2, 64) bf16: g per pixel, classes beyond K zero;   w2t64 (256, 64) bf16: W2 transposed, zero-padded.
+ * Everything else as mrfp_hrfp_tail_final2_bwd. */
 int mrfp_hrfp_tail_final2_bwd_rk(const mrfp_hrfp_plan_t* plan, const void* saved, const void* lut, const float* g,
                                  const float* w2, int K, void* g64, void* w2t64, float* g_w2, float* g_b2, void* stream);
-int mrfp_hrfp_bwd_rk(const mrfp_hrfp_plan_t* plan, const float* g_ocout, const void* g64, const void* w2t64,
-                     const float* const* gamma, const float* np_alpha, const float* np_eps, const float* np_mean,
-                     void* np_ws, const void* lut, const void* saved, float* g_xp, void* ws, void* stream);
 
 /* Backward of the reference's Upsample (network/mynn.py:114-119, bilinear, align_corners=True) at the up-sampling sites of
  * the tail (deepv3.py:356, :362), as a gather instead of ATen's atomicAdd scatter:

@@ -38,19 +38,14 @@ SIGNATURES = {
     "mrfp_hrfp_plan_write_luts": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_size_t]),
     "mrfp_hrfp_plan_stage": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_int, ctypes.POINTER(ctypes.c_int)]),
     "mrfp_hrfp_plan_set_fusion": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_int]),
+    "mrfp_hrfp_np_ws_bytes": (ctypes.c_size_t, [ctypes.c_int, ctypes.c_int]),
     "mrfp_hrfp_fwd": (ctypes.c_int, [ctypes.c_void_p, c_float_p, c_void_pp, c_void_pp, c_void_pp, c_void_pp,
                                      c_void_pp, ctypes.c_float, ctypes.c_float, c_float_p, c_float_p, c_float_p,
+                                     c_float_p, c_float_p, ctypes.c_void_p, c_float_p, c_float_p,
                                      ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p]),
-    "mrfp_hrfp_bwd": (ctypes.c_int, [ctypes.c_void_p, c_float_p, c_float_p, c_void_pp, ctypes.c_void_p,
-                                     ctypes.c_void_p, c_float_p, ctypes.c_void_p, ctypes.c_void_p]),
-    "mrfp_hrfp_np_ws_bytes": (ctypes.c_size_t, [ctypes.c_int, ctypes.c_int]),
-    "mrfp_hrfp_fwd_np": (ctypes.c_int, [ctypes.c_void_p, c_float_p, c_void_pp, c_void_pp, c_void_pp, c_void_pp,
-                                        c_void_pp, ctypes.c_float, ctypes.c_float, c_float_p, c_float_p, c_float_p,
-                                        c_float_p, ctypes.c_void_p, c_float_p, c_float_p,
-                                        ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p]),
-    "mrfp_hrfp_bwd_np": (ctypes.c_int, [ctypes.c_void_p, c_float_p, c_float_p, c_void_pp, c_float_p, c_float_p,
-                                        c_float_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, c_float_p,
-                                        ctypes.c_void_p, ctypes.c_void_p]),
+    "mrfp_hrfp_bwd": (ctypes.c_int, [ctypes.c_void_p, c_float_p, ctypes.c_int, ctypes.c_void_p, ctypes.c_void_p, c_void_pp,
+                                     c_float_p, c_float_p, c_float_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p,
+                                     c_float_p, ctypes.c_void_p, ctypes.c_void_p]),
     "mrfp_hrfp_plus_add": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, c_float_p, c_float_p,
                                           ctypes.c_void_p]),
     "mrfp_hrfp_plus_add_bilinear": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, c_float_p, ctypes.c_int,
@@ -59,15 +54,9 @@ SIGNATURES = {
                                                  ctypes.c_int, c_float_p, c_float_p, ctypes.c_int, c_float_p, ctypes.c_void_p]),
     "mrfp_hrfp_tail_final2_bwd": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, c_float_p, c_float_p,
                                                  ctypes.c_int, ctypes.c_void_p, c_float_p, c_float_p, ctypes.c_void_p]),
-    "mrfp_hrfp_bwd_nhwc": (ctypes.c_int, [ctypes.c_void_p, c_float_p, ctypes.c_void_p, c_void_pp, c_float_p, c_float_p,
-                                          c_float_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, c_float_p,
-                                          ctypes.c_void_p, ctypes.c_void_p]),
     "mrfp_hrfp_tail_final2_bwd_rk": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, c_float_p, c_float_p,
                                                     ctypes.c_int, ctypes.c_void_p, ctypes.c_void_p, c_float_p, c_float_p,
                                                     ctypes.c_void_p]),
-    "mrfp_hrfp_bwd_rk": (ctypes.c_int, [ctypes.c_void_p, c_float_p, ctypes.c_void_p, ctypes.c_void_p, c_void_pp, c_float_p,
-                                        c_float_p, c_float_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, c_float_p,
-                                        ctypes.c_void_p, ctypes.c_void_p]),
     "mrfp_add_f32": (ctypes.c_int, [c_float_p, c_float_p, c_float_p, ctypes.c_size_t, ctypes.c_void_p]),
     "mrfp_bilinear_bwd_table_bytes": (ctypes.c_size_t, [ctypes.c_int, ctypes.c_int]),
     "mrfp_bilinear_bwd_write_table": (ctypes.c_int, [ctypes.c_int, ctypes.c_int, ctypes.c_void_p, ctypes.c_size_t]),

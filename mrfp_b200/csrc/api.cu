@@ -24,7 +24,7 @@ int get_device_info(DeviceInfo* out) {
 }
 }  // namespace mrfp
 
-extern "C" int mrfp_version(void) { return 100; }
+extern "C" int mrfp_version(void) { return 101; }
 
 extern "C" const char* mrfp_strerror(int rc) {
   switch (rc) {

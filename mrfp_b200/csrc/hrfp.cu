@@ -1298,14 +1298,37 @@ int rankk_expand(const void* g64, const void* w2t, T* dA, long long npix, int C,
   }
 }
 
+// The gradient of OCout_dec in one of the forms of include/mrfp_b200.h (MRFP_DEC_GRAD_*): g is the fp32 NCHW tensor, the
+// NHWC tensor in the chain's element type, or the rank-K factor G with w2t = W2T.
+struct DecGrad {
+  int form;
+  const void* g;
+  const void* w2t;
+};
+
+// That gradient as the NHWC tensor dst (N, h/2, w/2, C) in the chain's element type.  Only the fp32 form is ever added to
+// what dst holds (FP32 mode); the other forms only overwrite it.
 template <typename T>
-int hrfp_backward(const mrfp_hrfp_plan* P, const float* g_ocout, const float* g_ocout_dec, const float* const* gamma,
+int materialise_dec(const mrfp_hrfp_plan* P, const DecGrad& dec, T* dst, bool accumulate, const DeviceInfo& di, cudaStream_t s) {
+  const HrfpStage& st = P->st[3];
+  const long long npix = (long long)P->N * st.oh * st.ow;
+  switch (dec.form) {
+    case MRFP_DEC_GRAD_F32:
+      run_nchw_to_nhwc<T>(static_cast<const float*>(dec.g), dst, P->N, st.cout, st.cout, st.oh * st.ow, accumulate,
+                          (double*)nullptr, true, s);
+      return MRFP_OK;
+    case MRFP_DEC_GRAD_NHWC:
+      MRFP_CUDA_TRY(cudaMemcpyAsync(dst, dec.g, (size_t)npix * st.cout * sizeof(T), cudaMemcpyDeviceToDevice, s));
+      return MRFP_OK;
+    default:
+      return rankk_expand<T>(dec.g, dec.w2t, dst, npix, st.cout, di, s);
+  }
+}
+
+template <typename T>
+int hrfp_backward(const mrfp_hrfp_plan* P, const float* g_ocout, const DecGrad& dec, const float* const* gamma,
                   const int* lut, const char* saved, float* g_xp, char* ws, cudaStream_t s, const DeviceInfo& di,
-                  const NpStem* np, const void* g_dec_nhwc, const void* rk_w2t = nullptr) {
-  // rk_w2t != nullptr: g_dec_nhwc is the RANK-K form of that gradient, G (N, h/2, w/2, 64) bf16 with W2T (C, 64) bf16 — it
-  // joins as one more k-block of the stage-4 dgrad and the (N, h/2, w/2, C) tensor never exists
-  // g_dec_nhwc: the gradient of OCout_dec already in the chain's layout (N, h/2, w/2, C) and element type — produced by
-  // the fused classifier tail (tail_final2.cu) — instead of the fp32 NCHW tensor g_ocout_dec
+                  const NpStem* np) {
   double* acc = reinterpret_cast<double*>(ws + P->acc_bwd_off);
   if (np && !g_ocout) np = nullptr;                      // no gradient through `x`: NP+ contributes nothing
   if (np) MRFP_CUDA_TRY(cudaMemsetAsync(np->psum, 0, (size_t)P->N * P->cin * sizeof(double), s));
@@ -1317,29 +1340,20 @@ int hrfp_backward(const mrfp_hrfp_plan* P, const float* g_ocout, const float* g_
   T* dA = nullptr;    // gradient wrt the stage output A_{k+1}, NHWC at (oh, ow)
   T* other = g1;
   bool at_end = true;     // where the last kernel that touched dA finished (the layout kernels walk front to back)
-  bool dec_joined = false;
   for (int k = kHrfpStages - 1; k >= 0; --k) {
     const HrfpStage& st = P->st[k];
-    const float* gin = (k == kHrfpStages - 1) ? g_ocout : (k == 3 ? g_ocout_dec : nullptr);
-    if (k == 3 && dec_joined) gin = nullptr;               // already added by the dgrad of stage 4
-    if (k == 3 && g_dec_nhwc && !dec_joined) {             // encoder-only backward: the tail's gradient IS dA_3
-      if (rk_w2t) {
-        int re = rankk_expand<T>(g_dec_nhwc, rk_w2t, g0, (long long)P->N * st.oh * st.ow, st.cout, di, s);
-        if (re) return re;
-      } else {
-        const size_t bytes = (size_t)P->N * st.oh * st.ow * st.cout * sizeof(T);
-        MRFP_CUDA_TRY(cudaMemcpyAsync(g0, g_dec_nhwc, bytes, cudaMemcpyDeviceToDevice, s));
-      }
-      dA = g0; other = g1; at_end = true;
-    }
-    if (gin) {
-      const int HW = st.oh * st.ow;
-      T* dst = dA ? dA : g0;
-      const bool np_here = np && k == kHrfpStages - 1;       // plane totals of g_ocout for the fused NP+ backward
-      run_nchw_to_nhwc<T>(gin, dst, P->N, st.cout_real, st.cout, HW, dA != nullptr, np_here ? np->psum : (double*)nullptr, true, s);
-      if (np_here)
+    if (k == kHrfpStages - 1 && g_ocout) {      // with the fused NP+ backward this pass also takes the plane totals of g_ocout
+      run_nchw_to_nhwc<T>(g_ocout, g0, P->N, st.cout_real, st.cout, st.oh * st.ow, false, np ? np->psum : (double*)nullptr, true, s);
+      if (np)
         launch_k(np_stem_coef_kernel<true>, dim3(1), dim3(256), 0, s, (const double*)np->psum, np->alpha, np->eps,
                  (const float*)np->mean, np->coef, (float*)nullptr, (float*)nullptr, P->N, P->cin, P->xh * P->xw);
+      dA = g0;
+    }
+    // The gradient of OCout_dec joins dA_3.  The tensor-core modes add it in the epilogue of stage 4's dgrad (below) when
+    // stages 7-4 ran; here it starts the encoder-only backward, or the FP32 mode adds it to dA_3.
+    if (k == 3 && dec.form != MRFP_DEC_GRAD_NONE && !(tc && dA)) {
+      int rd = materialise_dec<T>(P, dec, dA ? dA : g0, dA != nullptr, di, s);
+      if (rd) return rd;
       if (!dA) { dA = g0; other = g1; }
       at_end = true;
     }
@@ -1354,7 +1368,7 @@ int hrfp_backward(const mrfp_hrfp_plan* P, const float* g_ocout, const float* g_
     // over HBM: identity / down-sampling stages directly, up-sampling stages (up to 2 x 2 replicas per pixel) through an
     // extras stage.  (The fp32 OCout_dec gradient of the unfused tail is staged in the dA buffer, which the gathered dgrad
     // still reads: that case keeps the pass.)
-    const bool gathered = tc && (P->fuse & 2) && sizeof(T) == 2 && st.max_rep <= 2 && !(k == 4 && g_ocout_dec && !g_dec_nhwc) &&
+    const bool gathered = tc && (P->fuse & 2) && sizeof(T) == 2 && st.max_rep <= 2 && !(k == 4 && dec.form == MRFP_DEC_GRAD_F32) &&
                           !(st.max_rep > 1 && k == 4) &&
                           conv3x3_gather_supported(st.max_rep <= 1 ? 1 : 2, P->N, st.ch, st.cw, st.oh, st.ow, st.cout, st.cin, st.dil,
                                                    P->lut.data() + st.lo_h, P->lut.data() + st.lo_w);
@@ -1365,31 +1379,24 @@ int hrfp_backward(const mrfp_hrfp_plan* P, const float* g_ocout, const float* g_
     }
     // dgrad: conv of dY (cout channels) with the rotated / transposed kernel -> dA_prev (cin channels)
     if (tc) {
-      // stage 4's dgrad produces dA_3, which the gradient of OCout_dec has to join: convert that gradient into the
-      // buffer apply(4) has just finished reading and let the conv epilogue add it in fp32 (one rounding, and the
-      // read-modify-write pass over dA_3 disappears)
-      const T* add_src = nullptr;
+      // stage 4's dgrad produces dA_3, which the gradient of OCout_dec joins in the conv epilogue in fp32 (one rounding, and
+      // the read-modify-write pass over dA_3 disappears): the NHWC form as the add tile itself, the rank-K form as one more
+      // k-block of the gathered dgrad (G and W2T travel through its weight ring), any other case materialised into the
+      // buffer apply(4) has just finished reading
+      const void* add_src = nullptr;
       const void* rk = nullptr;
-      if (k == 4 && g_dec_nhwc && rk_w2t && gathered) {      // rank-K: G and W2T travel through the dgrad's weight ring
-        add_src = static_cast<const T*>(g_dec_nhwc);
-        rk = rk_w2t;
-        dec_joined = true;
-      } else if (k == 4 && g_dec_nhwc && rk_w2t) {           // ... unless the dgrad is the tap kernel: expand into the buffer
-        const HrfpStage& pv = P->st[3];                      // apply(4) has just finished reading
-        int re = rankk_expand<T>(g_dec_nhwc, rk_w2t, dA, (long long)P->N * pv.oh * pv.ow, pv.cout, di, s);
-        if (re) return re;
-        add_src = dA;
-        dec_joined = true;
-        at_end = true;
-      } else if (k == 4 && g_dec_nhwc) {
-        add_src = static_cast<const T*>(g_dec_nhwc);
-        dec_joined = true;
-      } else if (k == 4 && g_ocout_dec) {
-        const HrfpStage& pv = P->st[3];
-        run_nchw_to_nhwc<T>(g_ocout_dec, dA, P->N, pv.cout, pv.cout, pv.oh * pv.ow, false, (double*)nullptr, true, s);
-        add_src = dA;
-        dec_joined = true;
-        at_end = true;
+      if (k == 4 && dec.form != MRFP_DEC_GRAD_NONE) {
+        if (dec.form == MRFP_DEC_GRAD_NHWC) {
+          add_src = dec.g;
+        } else if (dec.form == MRFP_DEC_GRAD_RANK_K && gathered) {
+          add_src = dec.g;
+          rk = dec.w2t;
+        } else {
+          int rd = materialise_dec<T>(P, dec, dA, false, di, s);
+          if (rd) return rd;
+          add_src = dA;
+          at_end = true;
+        }
       }
       int rc;
       if (gathered)
@@ -1569,18 +1576,43 @@ extern "C" int mrfp_hrfp_plan_stage(const mrfp_hrfp_plan_t* P, int k, int* out7)
   return MRFP_OK;
 }
 
-static int hrfp_fwd_entry(const mrfp_hrfp_plan_t* P, const float* xp, const float* const* W, const float* const* gamma,
-                          const float* const* beta, float* const* running_mean, float* const* running_var, float momentum,
-                          float eps, const float* x_add, float* ocout, float* ocout_dec, const void* lut, void* saved,
-                          void* ws, void* stream, const NpStem* np) {
+extern "C" size_t mrfp_hrfp_np_ws_bytes(int N, int C) {
+  if (N <= 0 || C <= 0) return 0;
+  return (size_t)N * C * (sizeof(double) + sizeof(float2));
+}
+
+// NP+ call 1 folded into the chain when alpha, eps, mean and np_ws are all given, not folded (*np = nullptr) when none is
+static int np_stem_setup(const mrfp_hrfp_plan_t* P, const float* alpha, const float* eps, const float* mean, float* beta,
+                         void* np_ws, NpStem* stem, const NpStem** np) {
+  *np = nullptr;
+  if (!alpha && !eps && !mean && !np_ws) return MRFP_OK;
+  if (!alpha || !eps || !mean || !np_ws || ((uintptr_t)np_ws & 15)) return MRFP_ERR_NULL_POINTER;
+  stem->alpha = alpha; stem->eps = eps; stem->mean = const_cast<float*>(mean); stem->beta = beta;
+  stem->psum = reinterpret_cast<double*>(np_ws);
+  stem->coef = reinterpret_cast<float2*>(stem->psum + (size_t)P->N * P->cin);
+  *np = stem;
+  return MRFP_OK;
+}
+
+extern "C" int mrfp_hrfp_fwd(const mrfp_hrfp_plan_t* P, const float* xp, const float* const* W, const float* const* gamma,
+                             const float* const* beta, float* const* running_mean, float* const* running_var, float momentum,
+                             float eps, const float* x_add, const float* np_alpha, const float* np_eps, float* np_mean,
+                             float* np_beta, void* np_ws, float* ocout, float* ocout_dec, const void* lut, void* saved,
+                             void* ws, void* stream) {
   if (!P || P->magic != kPlanMagic) return MRFP_ERR_BAD_PLAN;
   if (!xp || !W || !gamma || !lut || !saved || !ws) return MRFP_ERR_NULL_POINTER;
+  NpStem stem;
+  const NpStem* np;
+  int rc = np_stem_setup(P, np_alpha, np_eps, np_mean, np_beta, np_ws, &stem, &np);
+  if (rc) return rc;
+  if (np && !ocout) return MRFP_ERR_NULL_POINTER;        // the fused form only exists for x = OCout + NP+(xp) ...
+  if (np && x_add) return MRFP_ERR_UNSUPPORTED;          // ... where NP+(xp) takes the place of x_add
   if (((uintptr_t)saved | (uintptr_t)ws | (uintptr_t)lut) & 255) return MRFP_ERR_WORKSPACE;
   const int last = ocout ? kHrfpStages : 4;
   for (int k = 0; k < last; ++k)
     if (!W[k] || !gamma[k]) return MRFP_ERR_NULL_POINTER;
   DeviceInfo di;
-  int rc = get_device_info(&di);
+  rc = get_device_info(&di);
   if (rc) return rc;
   cudaStream_t s = (cudaStream_t)stream;
   std::lock_guard<std::mutex> lock(P->mu);               // the plan's tensor-map cache
@@ -1591,107 +1623,45 @@ static int hrfp_fwd_entry(const mrfp_hrfp_plan_t* P, const float* xp, const floa
                              (const int*)lut, (char*)saved, (char*)ws, s, di, np);
 }
 
-static int hrfp_bwd_entry(const mrfp_hrfp_plan_t* P, const float* g_ocout, const float* g_ocout_dec,
-                          const float* const* gamma, const void* lut, const void* saved, float* g_xp, void* ws,
-                          void* stream, const NpStem* np, const void* g_dec_nhwc = nullptr, const void* rk_w2t = nullptr) {
+extern "C" int mrfp_hrfp_bwd(const mrfp_hrfp_plan_t* P, const float* g_ocout, int dec_form, const void* g_dec,
+                             const void* w2t64, const float* const* gamma, const float* np_alpha, const float* np_eps,
+                             const float* np_mean, void* np_ws, const void* lut, const void* saved, float* g_xp, void* ws,
+                             void* stream) {
   if (!P || P->magic != kPlanMagic) return MRFP_ERR_BAD_PLAN;
   if (!gamma || !lut || !saved || !g_xp || !ws) return MRFP_ERR_NULL_POINTER;
-  if (g_dec_nhwc && (g_ocout_dec || P->mode == MRFP_MATH_FP32 || ((uintptr_t)g_dec_nhwc & 15))) return MRFP_ERR_UNSUPPORTED;
-  if (rk_w2t && (!g_dec_nhwc || P->mode != MRFP_MATH_BF16 || ((uintptr_t)rk_w2t & 15))) return MRFP_ERR_UNSUPPORTED;
+  NpStem stem;
+  const NpStem* np;
+  int rc = np_stem_setup(P, np_alpha, np_eps, np_mean, nullptr, np_ws, &stem, &np);
+  if (rc) return rc;
+  switch (dec_form) {
+    case MRFP_DEC_GRAD_NONE:
+      break;
+    case MRFP_DEC_GRAD_F32:
+      if (!g_dec) return MRFP_ERR_NULL_POINTER;
+      break;
+    case MRFP_DEC_GRAD_NHWC:
+      if (!g_dec) return MRFP_ERR_NULL_POINTER;
+      if (P->mode == MRFP_MATH_FP32 || ((uintptr_t)g_dec & 15)) return MRFP_ERR_UNSUPPORTED;
+      break;
+    case MRFP_DEC_GRAD_RANK_K:      // w2t64 is (256, 64): the classifier tail, its producer, exists for 256 channels only
+      if (!g_dec || !w2t64) return MRFP_ERR_NULL_POINTER;
+      if (P->mode != MRFP_MATH_BF16 || P->st[3].cout != 256 || (((uintptr_t)g_dec | (uintptr_t)w2t64) & 15))
+        return MRFP_ERR_UNSUPPORTED;
+      break;
+    default:
+      return MRFP_ERR_UNSUPPORTED;
+  }
   if (((uintptr_t)saved | (uintptr_t)ws | (uintptr_t)lut) & 255) return MRFP_ERR_WORKSPACE;
   DeviceInfo di;
-  int rc = get_device_info(&di);
+  rc = get_device_info(&di);
   if (rc) return rc;
   cudaStream_t s = (cudaStream_t)stream;
   std::lock_guard<std::mutex> lock(P->mu);
+  const DecGrad dec = {dec_form, g_dec, w2t64};
   if (P->mode == MRFP_MATH_BF16)
-    return hrfp_backward<__nv_bfloat16>(P, g_ocout, g_ocout_dec, gamma, (const int*)lut, (const char*)saved, g_xp,
-                                        (char*)ws, s, di, np, g_dec_nhwc, rk_w2t);
-  return hrfp_backward<float>(P, g_ocout, g_ocout_dec, gamma, (const int*)lut, (const char*)saved, g_xp, (char*)ws, s, di,
-                              np, g_dec_nhwc);
-}
-
-extern "C" int mrfp_hrfp_fwd(const mrfp_hrfp_plan_t* P, const float* xp, const float* const* W,
-                             const float* const* gamma, const float* const* beta, float* const* running_mean,
-                             float* const* running_var, float momentum, float eps, const float* x_add, float* ocout,
-                             float* ocout_dec, const void* lut, void* saved, void* ws, void* stream) {
-  return hrfp_fwd_entry(P, xp, W, gamma, beta, running_mean, running_var, momentum, eps, x_add, ocout, ocout_dec, lut,
-                        saved, ws, stream, nullptr);
-}
-
-extern "C" int mrfp_hrfp_bwd(const mrfp_hrfp_plan_t* P, const float* g_ocout, const float* g_ocout_dec,
-                             const float* const* gamma, const void* lut, const void* saved, float* g_xp, void* ws,
-                             void* stream) {
-  return hrfp_bwd_entry(P, g_ocout, g_ocout_dec, gamma, lut, saved, g_xp, ws, stream, nullptr);
-}
-
-// ---- NP+ call 1 folded into the chain ----
-extern "C" size_t mrfp_hrfp_np_ws_bytes(int N, int C) {
-  if (N <= 0 || C <= 0) return 0;
-  return (size_t)N * C * (sizeof(double) + sizeof(float2));
-}
-
-static bool np_stem_setup(const mrfp_hrfp_plan_t* P, const float* alpha, const float* eps, float* mean, float* beta,
-                          void* np_ws, NpStem* np) {
-  if (!P || P->magic != kPlanMagic || !alpha || !eps || !mean || !np_ws || ((uintptr_t)np_ws & 15)) return false;
-  np->alpha = alpha; np->eps = eps; np->mean = mean; np->beta = beta;
-  np->psum = reinterpret_cast<double*>(np_ws);
-  np->coef = reinterpret_cast<float2*>(np->psum + (size_t)P->N * P->cin);
-  return true;
-}
-
-extern "C" int mrfp_hrfp_fwd_np(const mrfp_hrfp_plan_t* P, const float* xp, const float* const* W,
-                                const float* const* gamma, const float* const* beta, float* const* running_mean,
-                                float* const* running_var, float momentum, float eps, const float* np_alpha,
-                                const float* np_eps, float* np_mean, float* np_beta, void* np_ws, float* ocout,
-                                float* ocout_dec, const void* lut, void* saved, void* ws, void* stream) {
-  NpStem np;
-  if (!ocout) return MRFP_ERR_NULL_POINTER;              // the fused form only exists for x = OCout + NP+(xp)
-  if (!np_stem_setup(P, np_alpha, np_eps, np_mean, np_beta, np_ws, &np))
-    return (P && P->magic == kPlanMagic) ? MRFP_ERR_NULL_POINTER : MRFP_ERR_BAD_PLAN;
-  return hrfp_fwd_entry(P, xp, W, gamma, beta, running_mean, running_var, momentum, eps, nullptr, ocout, ocout_dec, lut,
-                        saved, ws, stream, &np);
-}
-
-extern "C" int mrfp_hrfp_bwd_np(const mrfp_hrfp_plan_t* P, const float* g_ocout, const float* g_ocout_dec,
-                                const float* const* gamma, const float* np_alpha, const float* np_eps,
-                                const float* np_mean, void* np_ws, const void* lut, const void* saved, float* g_xp,
-                                void* ws, void* stream) {
-  NpStem np;
-  if (!np_stem_setup(P, np_alpha, np_eps, const_cast<float*>(np_mean), nullptr, np_ws, &np))
-    return (P && P->magic == kPlanMagic) ? MRFP_ERR_NULL_POINTER : MRFP_ERR_BAD_PLAN;
-  return hrfp_bwd_entry(P, g_ocout, g_ocout_dec, gamma, lut, saved, g_xp, ws, stream, &np);
-}
-
-// The same two backward entry points with the gradient of OCout_dec given in the chain's own layout and element type
-// (N, h/2, w/2, C) — what mrfp_hrfp_tail_final2_bwd leaves — instead of an fp32 NCHW tensor.  np_* may all be NULL.
-extern "C" int mrfp_hrfp_bwd_nhwc(const mrfp_hrfp_plan_t* P, const float* g_ocout, const void* g_dec_nhwc,
-                                  const float* const* gamma, const float* np_alpha, const float* np_eps,
-                                  const float* np_mean, void* np_ws, const void* lut, const void* saved, float* g_xp,
-                                  void* ws, void* stream) {
-  if (!g_dec_nhwc) return MRFP_ERR_NULL_POINTER;
-  if (np_alpha || np_eps || np_mean || np_ws) {
-    NpStem np;
-    if (!np_stem_setup(P, np_alpha, np_eps, const_cast<float*>(np_mean), nullptr, np_ws, &np))
-      return (P && P->magic == kPlanMagic) ? MRFP_ERR_NULL_POINTER : MRFP_ERR_BAD_PLAN;
-    return hrfp_bwd_entry(P, g_ocout, nullptr, gamma, lut, saved, g_xp, ws, stream, &np, g_dec_nhwc);
-  }
-  return hrfp_bwd_entry(P, g_ocout, nullptr, gamma, lut, saved, g_xp, ws, stream, nullptr, g_dec_nhwc);
-}
-
-// ... and with that gradient in its RANK-K form (mrfp_hrfp_tail_final2_bwd_rk): g64 (N, h/2, w/2, 64) bf16 = the classifier's
-// incoming gradient per pixel, w2t (C, 64) bf16 = the classifier transposed; classes beyond K are zero in both.
-extern "C" int mrfp_hrfp_bwd_rk(const mrfp_hrfp_plan_t* P, const float* g_ocout, const void* g64, const void* w2t,
-                                const float* const* gamma, const float* np_alpha, const float* np_eps, const float* np_mean,
-                                void* np_ws, const void* lut, const void* saved, float* g_xp, void* ws, void* stream) {
-  if (!g64 || !w2t) return MRFP_ERR_NULL_POINTER;
-  if (np_alpha || np_eps || np_mean || np_ws) {
-    NpStem np;
-    if (!np_stem_setup(P, np_alpha, np_eps, const_cast<float*>(np_mean), nullptr, np_ws, &np))
-      return (P && P->magic == kPlanMagic) ? MRFP_ERR_NULL_POINTER : MRFP_ERR_BAD_PLAN;
-    return hrfp_bwd_entry(P, g_ocout, nullptr, gamma, lut, saved, g_xp, ws, stream, &np, g64, w2t);
-  }
-  return hrfp_bwd_entry(P, g_ocout, nullptr, gamma, lut, saved, g_xp, ws, stream, nullptr, g64, w2t);
+    return hrfp_backward<__nv_bfloat16>(P, g_ocout, dec, gamma, (const int*)lut, (const char*)saved, g_xp, (char*)ws, s, di,
+                                        np);
+  return hrfp_backward<float>(P, g_ocout, dec, gamma, (const int*)lut, (const char*)saved, g_xp, (char*)ws, s, di, np);
 }
 
 template <typename T>

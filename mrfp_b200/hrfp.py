@@ -21,16 +21,22 @@ MATH_FP32 = 0      # CUDA-core fp32 convolutions (tight parity mode)
 MATH_TF32 = 1      # tcgen05 kind::tf32, fp32 storage: the arithmetic of the reference's cuDNN convolutions (TF32 default)
 MATH_BF16 = 2      # tcgen05 kind::f16 on bf16 operands and bf16 storage, fp32 accumulation (default: half the HBM traffic)
 DEFAULT_WIDTHS = (64, 64, 128, 256)
+# form of the gradient of OCout_dec given to mrfp_hrfp_bwd (include/mrfp_b200.h: MRFP_DEC_GRAD_*)
+DEC_GRAD_NONE, DEC_GRAD_F32, DEC_GRAD_NHWC, DEC_GRAD_RANK_K = 0, 1, 2, 3
 
 
 def _stream_ptr(dev) -> int:
     return torch.cuda.current_stream(dev).cuda_stream
 
 
+def _ptr(t: Optional[torch.Tensor]):
+    return None if t is None else t.data_ptr()
+
+
 def _ptr_array(tensors: Sequence[Optional[torch.Tensor]]):
     arr = (ctypes.c_void_p * len(tensors))()
     for i, t in enumerate(tensors):
-        arr[i] = None if t is None else t.data_ptr()
+        arr[i] = _ptr(t)
     return arr
 
 
@@ -107,13 +113,39 @@ def get_plan(n, cin, xh, xw, h, w, device, math_mode=MATH_BF16, widths=DEFAULT_W
     return p
 
 
+class DecGradSlot:
+    """The gradient of a lazy OCout_dec, parked by the backward of its consumer until the chain's backward takes it:
+    the fp32 NCHW gradients of hrfp_plus_add / hrfp_plus_add_upsampled (summed), or one form left by the classifier tail
+    (an NHWC tensor, or the rank-K factors g and w2t)."""
+    __slots__ = ("form", "g", "w2t")
+
+    def __init__(self):
+        self.form, self.g, self.w2t = DEC_GRAD_NONE, None, None
+
+    def add_f32(self, g):
+        if self.form not in (DEC_GRAD_NONE, DEC_GRAD_F32):
+            raise _lib.MrfpError("OCout_dec was consumed both by the fused classifier tail and by a plain HRFP+ add")
+        self.form, self.g = DEC_GRAD_F32, (g if self.g is None else self.g + g)
+
+    def set_tail(self, form, g, w2t=None):
+        if self.form != DEC_GRAD_NONE:
+            raise _lib.MrfpError("OCout_dec handle consumed twice")
+        self.form, self.g, self.w2t = form, g, w2t
+
+    def take(self):
+        """(form, g, w2t), leaving the slot empty."""
+        out = (self.form, self.g, self.w2t)
+        self.__init__()
+        return out
+
+
 class HrfpDec:
     """OCout_dec left in the chain's saved state instead of being materialised as a (N,256,h/2,w/2) fp32 tensor:
     `hrfp_plus_add(dec1_up, handle)` produces `dec1_up + OCout_dec` in one pass and routes the gradient back."""
 
-    def __init__(self, plan, saved, token, mail):
+    def __init__(self, plan, saved, token, slot):
         self.plan, self.saved, self.token = plan, saved, token
-        self.mail = mail          # {"g": gradient parked by the add's backward}; shared with the chain's ctx (no cycle)
+        self.slot = slot          # DecGradSlot shared with the chain's ctx (a reference to ctx would be a cycle)
 
     @property
     def shape(self):
@@ -143,6 +175,7 @@ class _HrfpFn(torch.autograd.Function):
         rma = _ptr_array(rmeans) if rmeans is not None else None
         rva = _ptr_array(rvars) if rvars is not None else None
         ctx.np = None
+        np_ptrs = (None,) * 5          # np_alpha, np_eps, np_mean, np_beta, np_ws: NP+ not folded in
         if np_draws is not None:
             if x_add is not None or not want_out:
                 raise _lib.MrfpError("np_draws folds NP+(xp) into OCout + x: it needs want_out and no x_add")
@@ -151,37 +184,28 @@ class _HrfpFn(torch.autograd.Function):
             np_eps = np_draws[1].reshape(n, c).to(torch.float32).contiguous()
             np_mean = torch.empty((n, c), dtype=torch.float32, device=dev)
             np_ws = _lib.scratch(dev, lib.mrfp_hrfp_np_ws_bytes(n, c), "hrfp_np")      # per-call scratch (both directions)
-            with torch.cuda.device(dev):
-                rc = lib.mrfp_hrfp_fwd_np(plan.handle, xp_c.data_ptr(), wa, ga, ba, rma, rva, momentum, eps,
-                                          np_alpha.data_ptr(), np_eps.data_ptr(), np_mean.data_ptr(), None,
-                                          np_ws.data_ptr(), ocout.data_ptr(),
-                                          None if ocdec is None else ocdec.data_ptr(),
-                                          plan.lut.data_ptr(), saved.data_ptr(), ws.data_ptr(), _stream_ptr(dev))
-            _lib.check(rc, "mrfp_hrfp_fwd_np")
+            np_ptrs = (np_alpha.data_ptr(), np_eps.data_ptr(), np_mean.data_ptr(), None, np_ws.data_ptr())
             ctx.np = (np_alpha, np_eps, np_mean)
-        else:
-            with torch.cuda.device(dev):
-                rc = lib.mrfp_hrfp_fwd(plan.handle, xp_c.data_ptr(), wa, ga, ba, rma, rva, momentum, eps,
-                                       None if xa is None else xa.data_ptr(),
-                                       None if ocout is None else ocout.data_ptr(),
-                                       None if ocdec is None else ocdec.data_ptr(),
-                                       plan.lut.data_ptr(), saved.data_ptr(), ws.data_ptr(), _stream_ptr(dev))
-            _lib.check(rc, "mrfp_hrfp_fwd")
+        with torch.cuda.device(dev):
+            rc = lib.mrfp_hrfp_fwd(plan.handle, xp_c.data_ptr(), wa, ga, ba, rma, rva, momentum, eps, _ptr(xa), *np_ptrs,
+                                   _ptr(ocout), _ptr(ocdec), plan.lut.data_ptr(), saved.data_ptr(), ws.data_ptr(),
+                                   _stream_ptr(dev))
+        _lib.check(rc, "mrfp_hrfp_fwd")
         ctx.plan = plan
         ctx.saved_buf = saved
         ctx.gammas = [g for g in gammas]       # gamma is read again in backward: it must still be the forward's
         ctx.gamma_versions = [g._version for g in gammas]
         ctx.has_add = x_add is not None
         ctx.want_out, ctx.want_dec = want_out, want_dec
-        ctx.mail = None
+        ctx.slot = None
         outs = []
         if want_out:
             outs.append(ocout)
         if want_dec:
             if lazy_dec:
                 token = torch.zeros(1, dtype=torch.float32, device=dev)    # carries the autograd edge only
-                ctx.mail = {"g": None}
-                holder.append(HrfpDec(plan, saved, token, ctx.mail))
+                ctx.slot = DecGradSlot()
+                holder.append(HrfpDec(plan, saved, token, ctx.slot))
                 outs.append(token)
             else:
                 outs.append(ocdec)
@@ -200,15 +224,10 @@ class _HrfpFn(torch.autograd.Function):
         gi = iter(grads)
         g_out = next(gi) if ctx.want_out else None
         g_dec = next(gi) if ctx.want_dec else None
-        g_dec_nhwc = None
-        g_rk = None
-        if ctx.mail is not None:             # the real gradient was parked by the tail's backward
-            g_dec = ctx.mail["g"]
-            ctx.mail["g"] = None
-            g_dec_nhwc = ctx.mail.pop("g_nhwc", None)      # fused classifier tail: already NHWC in the chain's element type
-            g_rk = ctx.mail.pop("g_rk", None)              # ... or its rank-K form (g64, w2t64)
-            if (g_dec_nhwc is not None or g_rk is not None) and g_dec is not None:
-                raise _lib.MrfpError("OCout_dec was consumed both by the fused classifier tail and by a plain HRFP+ add")
+        if ctx.slot is not None:             # lazy OCout_dec: its consumer parked the real gradient
+            form, g_dec, w2t = ctx.slot.take()
+        else:
+            form, w2t = (DEC_GRAD_NONE if g_dec is None else DEC_GRAD_F32), None
         dev = plan.device
         g_out_c = g_out.contiguous() if g_out is not None else None
         g_dec_c = g_dec.contiguous() if g_dec is not None else None
@@ -217,34 +236,14 @@ class _HrfpFn(torch.autograd.Function):
             g_xp = torch.empty((plan.n, plan.cin, plan.xh, plan.xw), dtype=torch.float32, device=dev)
             ga = _ptr_array(ctx.gammas)
             ws = plan.workspace()
+            np_ptrs = (None,) * 4          # np_alpha, np_eps, np_mean, np_ws
+            if ctx.np is not None:         # gradient through NP+(xp) joins in the chain's last pass
+                np_ws = _lib.scratch(dev, lib.mrfp_hrfp_np_ws_bytes(plan.n, plan.cin), "hrfp_np")
+                np_ptrs = tuple(t.data_ptr() for t in ctx.np + (np_ws,))
             with torch.cuda.device(dev):
-                if g_rk is not None:
-                    a_, e_, m_ = ctx.np if ctx.np is not None else (None, None, None)
-                    w_ = _lib.scratch(dev, lib.mrfp_hrfp_np_ws_bytes(plan.n, plan.cin), "hrfp_np") if ctx.np is not None else None
-                    rc = lib.mrfp_hrfp_bwd_rk(plan.handle, None if g_out_c is None else g_out_c.data_ptr(), g_rk[0].data_ptr(),
-                                              g_rk[1].data_ptr(), ga, None if a_ is None else a_.data_ptr(),
-                                              None if e_ is None else e_.data_ptr(), None if m_ is None else m_.data_ptr(),
-                                              None if w_ is None else w_.data_ptr(), plan.lut.data_ptr(), ctx.saved_buf.data_ptr(),
-                                              g_xp.data_ptr(), ws.data_ptr(), _stream_ptr(dev))
-                elif g_dec_nhwc is not None:
-                    a_, e_, m_ = ctx.np if ctx.np is not None else (None, None, None)
-                    w_ = _lib.scratch(dev, lib.mrfp_hrfp_np_ws_bytes(plan.n, plan.cin), "hrfp_np") if ctx.np is not None else None
-                    rc = lib.mrfp_hrfp_bwd_nhwc(plan.handle, None if g_out_c is None else g_out_c.data_ptr(), g_dec_nhwc.data_ptr(),
-                                                ga, None if a_ is None else a_.data_ptr(), None if e_ is None else e_.data_ptr(),
-                                                None if m_ is None else m_.data_ptr(), None if w_ is None else w_.data_ptr(),
-                                                plan.lut.data_ptr(), ctx.saved_buf.data_ptr(), g_xp.data_ptr(), ws.data_ptr(),
-                                                _stream_ptr(dev))
-                elif ctx.np is not None:      # gradient through NP+(xp) joins in the chain's last pass
-                    a_, e_, m_ = ctx.np
-                    w_ = _lib.scratch(dev, lib.mrfp_hrfp_np_ws_bytes(plan.n, plan.cin), "hrfp_np")
-                    rc = lib.mrfp_hrfp_bwd_np(plan.handle, None if g_out_c is None else g_out_c.data_ptr(),
-                                              None if g_dec_c is None else g_dec_c.data_ptr(), ga, a_.data_ptr(),
-                                              e_.data_ptr(), m_.data_ptr(), w_.data_ptr(), plan.lut.data_ptr(),
-                                              ctx.saved_buf.data_ptr(), g_xp.data_ptr(), ws.data_ptr(), _stream_ptr(dev))
-                else:
-                    rc = lib.mrfp_hrfp_bwd(plan.handle, None if g_out_c is None else g_out_c.data_ptr(),
-                                           None if g_dec_c is None else g_dec_c.data_ptr(), ga, plan.lut.data_ptr(),
-                                           ctx.saved_buf.data_ptr(), g_xp.data_ptr(), ws.data_ptr(), _stream_ptr(dev))
+                rc = lib.mrfp_hrfp_bwd(plan.handle, _ptr(g_out_c), form, _ptr(g_dec_c), _ptr(w2t), ga, *np_ptrs,
+                                       plan.lut.data_ptr(), ctx.saved_buf.data_ptr(), g_xp.data_ptr(), ws.data_ptr(),
+                                       _stream_ptr(dev))
             _lib.check(rc, "mrfp_hrfp_bwd")
         g_add = g_out_c if (ctx.has_add and ctx.needs_input_grad[1]) else None
         ctx.saved_buf = None
@@ -315,12 +314,12 @@ class _PlusAddFusedFn(torch.autograd.Function):
             rc = lib.mrfp_hrfp_plus_add(plan.handle, handle.saved.data_ptr(), plan.lut.data_ptr(), a.data_ptr(),
                                         out.data_ptr(), _stream_ptr(a.device))
         _lib.check(rc, "mrfp_hrfp_plus_add")
-        ctx.mail = handle.mail
+        ctx.slot = handle.slot
         return out
 
     @staticmethod
     def backward(ctx, g):
-        ctx.mail["g"] = g if ctx.mail["g"] is None else ctx.mail["g"] + g
+        ctx.slot.add_f32(g)
         return g, torch.zeros(1, dtype=torch.float32, device=g.device), None
 
 
@@ -345,13 +344,13 @@ class _PlusAddUpFn(torch.autograd.Function):
             rc = lib.mrfp_hrfp_plus_add_bilinear(plan.handle, handle.saved.data_ptr(), plan.lut.data_ptr(), a.data_ptr(),
                                                  a.shape[2], a.shape[3], out.data_ptr(), _stream_ptr(a.device))
         _lib.check(rc, "mrfp_hrfp_plus_add_bilinear")
-        ctx.mail = handle.mail
+        ctx.slot = handle.slot
         ctx.lo_shape = tuple(a.shape)
         return out
 
     @staticmethod
     def backward(ctx, g):
-        ctx.mail["g"] = g if ctx.mail["g"] is None else ctx.mail["g"] + g
+        ctx.slot.add_f32(g)
         g_lo = None
         if ctx.needs_input_grad[0]:
             from .bilinear import bilinear_up_backward          # gather form of ATen's scatter (csrc/bilinear.cu)
@@ -420,26 +419,24 @@ class _TailFinal2Fn(torch.autograd.Function):
         g_t = bilinear_up_backward(gc, ctx.lo) if ctx.needs_input_grad[0] else None
         g_w2 = torch.empty((k, c), dtype=torch.float32, device=g.device)
         g_b2 = torch.empty((k,), dtype=torch.float32, device=g.device)
-        if handle.mail.get("g_nhwc") is not None or handle.mail.get("g_rk") is not None or handle.mail.get("g") is not None:
-            raise _lib.MrfpError("OCout_dec handle consumed twice")
         if os.environ.get("MRFP_TAIL_RANKK", "1") != "0":
-            # rank-K form: W2^T g joins the chain as its two factors (include/mrfp_b200.h: mrfp_hrfp_bwd_rk)
+            # rank-K form: W2^T g joins the chain as its two factors (include/mrfp_b200.h: MRFP_DEC_GRAD_RANK_K)
             g64 = torch.empty((n, oh, ow, 64), dtype=torch.bfloat16, device=g.device)
             w2t = torch.empty((c, 64), dtype=torch.bfloat16, device=g.device)
+            handle.slot.set_tail(DEC_GRAD_RANK_K, g64, w2t)
             with torch.cuda.device(g.device):
                 rc = lib.mrfp_hrfp_tail_final2_bwd_rk(plan.handle, handle.saved.data_ptr(), plan.lut.data_ptr(), gc.data_ptr(),
                                                       ctx.w2.data_ptr(), k, g64.data_ptr(), w2t.data_ptr(), g_w2.data_ptr(),
                                                       g_b2.data_ptr(), _stream_ptr(g.device))
             _lib.check(rc, "mrfp_hrfp_tail_final2_bwd_rk")
-            handle.mail["g_rk"] = (g64, w2t)
         else:
             g_nhwc = torch.empty((n, oh, ow, c), dtype=torch.bfloat16, device=g.device)
+            handle.slot.set_tail(DEC_GRAD_NHWC, g_nhwc)
             with torch.cuda.device(g.device):
                 rc = lib.mrfp_hrfp_tail_final2_bwd(plan.handle, handle.saved.data_ptr(), plan.lut.data_ptr(), gc.data_ptr(),
                                                    ctx.w2.data_ptr(), k, g_nhwc.data_ptr(), g_w2.data_ptr(), g_b2.data_ptr(),
                                                    _stream_ptr(g.device))
             _lib.check(rc, "mrfp_hrfp_tail_final2_bwd")
-            handle.mail["g_nhwc"] = g_nhwc
         return (g_t, g_w2.reshape(ctx.wshape) if ctx.needs_input_grad[1] else None,
                 g_b2 if (ctx.has_bias and ctx.needs_input_grad[2]) else None,
                 torch.zeros(1, dtype=torch.float32, device=g.device), None)

@@ -219,7 +219,7 @@ def test_classifier_tail_at_benchmarked_shape():
     chain (so the difference is the bf16 rounding of the classifier operands only), the gradient that joins the chain
     against W2^T g rounded to bf16."""
     import torch.nn.functional as F
-    from mrfp_b200.hrfp import hrfp_chain, hrfp_plus_add_upsampled, hrfp_plus_final2
+    from mrfp_b200.hrfp import DEC_GRAD_NHWC, DEC_GRAD_RANK_K, hrfp_chain, hrfp_plus_add_upsampled, hrfp_plus_final2
     n, k = 2, 19
     ws, gs = make_hrfp_params(31)
     gen = torch.Generator(device="cuda").manual_seed(32)
@@ -238,9 +238,11 @@ def test_classifier_tail_at_benchmarked_shape():
     dec = chain()
     out = hrfp_plus_final2(da, final2, dec)
     out.backward(g)
-    g_nhwc = dec.mail.get("g_nhwc")                                # (N, h/2, w/2, 256) bf16: the rank-K gradient of OCout_dec
-    if g_nhwc is None and dec.mail.get("g_rk") is not None:        # ... left as its two factors (mrfp_hrfp_tail_final2_bwd_rk)
-        g64, w2t = dec.mail["g_rk"]
+    slot = dec.slot
+    assert slot.form in (DEC_GRAD_NHWC, DEC_GRAD_RANK_K), slot.form    # the tail's backward parked its gradient
+    g_nhwc = slot.g if slot.form == DEC_GRAD_NHWC else None        # (N, h/2, w/2, 256) bf16: the gradient of OCout_dec
+    if slot.form == DEC_GRAD_RANK_K:                               # ... left as its two factors (mrfp_hrfp_tail_final2_bwd_rk)
+        g64, w2t = slot.g, slot.w2t
         assert float(g64[..., k:].abs().max()) == 0.0 and float(w2t[:, k:].abs().max()) == 0.0
         assert torch.equal(g64[..., :k], g.bfloat16().permute(0, 2, 3, 1)) and torch.equal(w2t[:, :k], final2.weight.detach().reshape(k, 256).bfloat16().t())
         g_nhwc = g64.double() @ w2t.double().t()

@@ -454,7 +454,7 @@ def test_tail_fused_through_the_classifier_equals_the_unfused_tail(geom):
 @pytest.mark.parametrize("want_out", [True, False])
 def test_rank_k_form_of_the_tail_gradient_in_the_full_chain(geom, fuse, want_out, monkeypatch):
     """The gradient of OCout_dec out of the fused classifier tail is W2^T g (rank K): by default it joins the chain as its two
-    factors and the stage-4 dgrad accumulates their product as one more k-block (mrfp_hrfp_tail_final2_bwd_rk + mrfp_hrfp_bwd_rk,
+    factors and the stage-4 dgrad accumulates their product as one more k-block (mrfp_hrfp_tail_final2_bwd_rk + MRFP_DEC_GRAD_RANK_K,
     conv_gather.cu ADD == 2) — against the materialised (N, h/2, w/2, 256) bf16 tensor added in that dgrad's epilogue
     (MRFP_TAIL_RANKK=0) and against the unfused tail.  Without the fused BN backward (fuse bit 1 off: fuse 0, 1) the stage-4
     dgrad is the tap kernel and the product is expanded into the dA buffer first; in the encoder-only backward
